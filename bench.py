@@ -2,6 +2,7 @@
 """Headline benchmark: output Mpix/s of the panorama -> plane hot path (8K equirect -> 1920x1080).
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this framework (CUDA)
+    python bench.py ... --dump-outputs DIR                         # + a fixed sample of the last timed step's outputs
     python bench.py --impl reference [--steps K] [--warmup W]      # CPU reference arm
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W     # N > 1, one rank per GPU
@@ -27,6 +28,11 @@ e2e.frac_of_transfer_ceiling   time of the bare page-locked copies of the same b
 e2e_files  JPEG file in -> 12 JPEG files out per image (8.6 MB instead of 150 MB over PCIe), every rank, aggregate.
 parity   every rank renders one view of one of ITS OWN seeds and compares it with the CPU oracle outside the timed
          regions (bit-exact when the host's NumPy takes the SVML path the kernel restates, else >= 96 % of pixels).
+
+--dump-outputs DIR  rank 0 writes what the last timed step computed, the [BATCH, yaw, pitch, H, W, 3] u8 views of its 32
+         images (2.4 GB), at DUMP_PIXELS fixed pixel positions (seeded, the same in every view) as float32:
+         DIR/views.npy [32, 4, 3, DUMP_PIXELS, 3] and the positions DIR/views_yx.npy [DUMP_PIXELS, 2] (row, column).  The
+         inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -45,6 +51,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True  # the tree may be read-only: the imports below leave no __pycache__ in it
 
 METRIC = "output Mpix/s (8K equirect -> 1920x1080)"
 UNIT = "Mpix/s"
@@ -60,6 +67,7 @@ B_ALG_PER_IMAGE = 3 * PX_PER_IMAGE + 3 * N_T_C2  # 141,009,384 bytes = 5.667 B /
 BATCH = 32  # images per GPU per step (configs[2]: 256 images over 8 GPUs)
 H2D_PER_IMAGE = WP * HP * 3
 D2H_PER_IMAGE = PX_PER_IMAGE * 3
+DUMP_PIXELS = 8192  # per view for --dump-outputs: 32 x 12 x 8192 x 3 float32 = 37.7 MB
 
 
 def workload_config(extra=None):
@@ -343,6 +351,8 @@ def run_b200_arm(args, rank: int, local_rank: int, world: int):
     torch.cuda.synchronize()
     ms_local = timed_steps(args.steps)
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, d_out, Path(args.dump_outputs))
     barrier()
     ms_total = max_over_ranks(ms_local)
     launches = proj.launches - launches0
@@ -501,6 +511,16 @@ def run_b200_arm(args, rank: int, local_rank: int, world: int):
         b.free()
     proj.close()
     ranks.close()
+
+
+def dump_outputs(torch, d_out, out_dir: Path):
+    """--dump-outputs: the views of the last timed step at DUMP_PIXELS fixed pixel positions (see the module docstring)."""
+    flat = np.sort(np.random.default_rng(0).choice(H * W, DUMP_PIXELS, replace=False))
+    idx = torch.from_numpy(flat).to(d_out.device)
+    views = d_out.view(BATCH, len(YAWS), len(PITCHES), H * W, 3).index_select(3, idx)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "views.npy", views.float().cpu().numpy())
+    np.save(out_dir / "views_yx.npy", np.stack([flat // W, flat % W], axis=1).astype(np.float32))
 
 
 def transfer_ceiling(torch, dev, pin_in, pin_out, h2d_bytes, d2h_bytes, barrier, max_over_ranks, steps=2):
@@ -785,7 +805,11 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the files-to-files (JPEG in, JPEG out) side measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last timed step's outputs as DIR/*.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

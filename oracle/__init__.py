@@ -19,4 +19,5 @@ ref_port     two-pass NumPy + cv2.remap restatement (what the reference executes
 fixedpoint   cv2-free integer model of ``cv2.remap(INTER_LINEAR, BORDER_CONSTANT)`` and the
              single-pass per-pixel restatement the CUDA kernel follows (SURVEY Appendix A)
 synth        deterministic synthetic panoramas (noise / smooth / coords)
+golden       reads and writes the golden vectors under ``tests/golden/``
 """

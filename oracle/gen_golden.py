@@ -28,7 +28,7 @@ GOLDEN = ROOT / "tests" / "golden"
 REF_FILE = Path("/root/reference/app/panorama_to_plane-pitch.py")
 
 sys.path.insert(0, str(ROOT))
-from oracle import synth  # noqa: E402
+from oracle import golden, synth  # noqa: E402
 
 
 def load_reference():
@@ -97,11 +97,12 @@ def main():
     yaws, pitches = [0, 90, 180, 270], [30, 60, 90]
     W, H, fov, Wp, Hp = 240, 135, 120, 1024, 512
     U, V = ref_maps(ref, pitches, W, H, fov, Wp, Hp)
-    np.savez_compressed(
+    golden.save(
         GOLDEN / "c2_small.npz",
-        out_noise=ref_views(ref, pano("noise", Wp, Hp), yaws, pitches, W, H, fov),
-        out_smooth=ref_views(ref, pano("smooth", Wp, Hp), yaws, pitches, W, H, fov),
-        U=U, V=V, yaws=yaws, pitches=pitches, W=W, H=H, fov=fov, Wp=Wp, Hp=Hp, seed=0,
+        dict(out_noise=ref_views(ref, pano("noise", Wp, Hp), yaws, pitches, W, H, fov),
+             out_smooth=ref_views(ref, pano("smooth", Wp, Hp), yaws, pitches, W, H, fov),
+             U=U, V=V, yaws=yaws, pitches=pitches, W=W, H=H, fov=fov, Wp=Wp, Hp=Hp, seed=0),
+        from_maps=("out_noise", "out_smooth"),
     )
 
     # C5 scaled: cube faces incl. pole pitches (function-level 0/180 and CLI-legal 1/179)
@@ -130,8 +131,8 @@ def main():
     out = ref_views(ref, p, [0], [5, 175], W, H, fov)
     U, V = ref_maps(ref, [5, 175], W, H, fov, Wp, Hp)
     nan_px = np.argwhere(np.isnan(U) | np.isnan(V))
-    np.savez_compressed(GOLDEN / "nan_case.npz", out=out, nan_px=nan_px, yaws=[0], pitches=[5, 175],
-                        W=W, H=H, fov=fov, Wp=Wp, Hp=Hp, kind="smooth", seed=0)
+    golden.save(GOLDEN / "nan_case.npz", dict(out=out, nan_px=nan_px, yaws=[0], pitches=[5, 175],
+                                              W=W, H=H, fov=fov, Wp=Wp, Hp=Hp, kind="smooth", seed=0), dx=("out",))
 
     if args.full:
         # full-size configs: hashes only (bit-exactness of the CPU oracle at BASELINE sizes)

@@ -13,7 +13,7 @@ import numpy as np
 import pytest
 
 from oracle import fixedpoint as fp
-from oracle import ref_port, synth
+from oracle import golden, ref_port, synth
 
 pytestmark = pytest.mark.gpu
 
@@ -29,7 +29,7 @@ MIRROR_DEFAULT = 2
 
 
 def load(golden_dir, name):
-    return np.load(golden_dir / name, allow_pickle=False)
+    return golden.load(golden_dir / name)
 
 
 def ulp_diff(a, b):
@@ -130,7 +130,7 @@ def test_g2_coordinates_bit_exact_with_numpy_exact_trig(proj, golden_dir, name):
     golden maps -> every U and V of the reference's pitch maps is reproduced bit for bit."""
     g = load(golden_dir, name)
     Wp, Hp, W, H, fov = (int(g[k]) for k in ("Wp", "Hp", "W", "H", "fov"))
-    pitches = g["pitches"] if "pitches" in g.files else g["map_pitches"]
+    pitches = g["pitches"] if "pitches" in g else g["map_pitches"]
     for j, p in enumerate(pitches):
         U, V = proj.coords(W, H, fov, int(p), Wp, Hp)
         assert np.array_equal(U.view(np.uint32), g["U"][j].view(np.uint32)), int(p)
@@ -151,7 +151,7 @@ def minimax_trig(pkg, proj):
 def test_g2_coordinates_within_fp32_tolerance(proj, golden_dir, name, minimax_trig):
     g = load(golden_dir, name)
     Wp, Hp, W, H, fov = (int(g[k]) for k in ("Wp", "Hp", "W", "H", "fov"))
-    pitches = g["pitches"] if "pitches" in g.files else g["map_pitches"]
+    pitches = g["pitches"] if "pitches" in g else g["map_pitches"]
     report = {}
     for j, p in enumerate(pitches):
         U, V = proj.coords(W, H, fov, int(p), Wp, Hp)

@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 from oracle import fixedpoint as fp
-from oracle import ref_port, synth
+from oracle import golden, ref_port, synth
 
 
 def sha(a):
@@ -31,7 +31,7 @@ def manifest(golden_dir):
 
 
 def load(golden_dir, name):
-    return np.load(golden_dir / name, allow_pickle=False)
+    return golden.load(golden_dir / name)
 
 
 def test_synthetic_panoramas_are_reproducible(manifest):
@@ -41,6 +41,19 @@ def test_synthetic_panoramas_are_reproducible(manifest):
         if Wp * Hp > 2048 * 1024:
             continue  # the big ones are covered by the hash tests below
         assert sha(synth.make(kind, Wp, Hp, int(seed[1:]))) == want, key
+
+
+def test_golden_files_are_small_and_decode_exactly(golden_dir, tmp_path):
+    """Every golden file stays under 1 MB; a file written with the encodings of ``oracle/golden.py`` loads back to exactly
+    the arrays it was given, and views that the stored maps do not reproduce are refused."""
+    for f in golden_dir.iterdir():
+        assert f.stat().st_size < 1 << 20, f.name
+    g = load(golden_dir, "c2_small.npz")
+    golden.save(tmp_path / "ok.npz", g, dx=("out_smooth",), from_maps=("out_noise",))
+    bad = dict(g, out_noise=g["out_noise"].copy())
+    bad["out_noise"][1, 2, 5, 7, 0] ^= 1
+    with pytest.raises(ValueError, match=r"views \(yaw index, pitch index\) \[\[1, 2\]\] differ"):
+        golden.save(tmp_path / "bad.npz", bad, from_maps=("out_noise",))
 
 
 def test_remap_model_matches_cv2_on_random_maps():
