@@ -30,6 +30,7 @@ from .panorama_to_plane_pitch import (  # noqa: E402
     scatter_upload,
     set_device,
     set_devices,
+    set_png_formats,
     yaw_mapping_cache,
 )
 from ._lib import P2PError, PitchConsts  # noqa: E402

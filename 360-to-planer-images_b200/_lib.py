@@ -67,6 +67,8 @@ SIGNATURES = {
     "p2p_decode_jpeg": (_i, [_vp, _i, _u8p, _sz, _u8p, _sz, _sz]),
     "p2p_png_probe": (_i, [_u8p, _sz, C.POINTER(_i), C.POINTER(_i)]),
     "p2p_png_decode_host": (_i, [_u8p, _sz, _u8p, _sz, _sz, C.POINTER(C.c_uint64)]),
+    "p2p_png_probe_ex": (_i, [_u8p, _sz, _i, C.POINTER(_i), C.POINTER(_i)]),
+    "p2p_png_decode_host_ex": (_i, [_u8p, _sz, _i, _u8p, _sz, _sz, C.POINTER(C.c_uint64)]),
     "p2p_upload_pano_png": (_i, [_vp, _i, _u8p, _sz, C.POINTER(_i), C.POINTER(_i)]),
     "p2p_decode_png": (_i, [_vp, _i, _u8p, _sz, _u8p, _sz, _sz]),
     "p2p_sync": (_i, [_vp, _i]),
@@ -90,6 +92,7 @@ OPT_GPU_HUFFMAN, OPT_GPU_HUFFMAN_COUNT = 9, 10
 OPT_SEG_CHUNKS = 11
 OPT_SEAM_WRAP = 12
 OPT_HOST_WAIT = 13
+OPT_PNG_FORMATS = 14
 
 _lib = None
 

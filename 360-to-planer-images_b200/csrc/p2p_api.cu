@@ -188,6 +188,10 @@ int p2p_set_option(p2p_ctx *ctx, int key, int value) {
             if (value != 0 && value != 1) return fail(ctx, P2P_ERR_INVALID, "host_wait must be 0 or 1");
             ctx->opt_host_wait.store(value);
             return P2P_OK;
+        case P2P_OPT_PNG_FORMATS:
+            if (value != 0 && value != 1) return fail(ctx, P2P_ERR_INVALID, "png_formats must be 0 or 1");
+            ctx->opt_png_formats.store(value);
+            return P2P_OK;
         case P2P_OPT_GPU_HUFFMAN:
             if (value < 0 || value > 3) return fail(ctx, P2P_ERR_INVALID, "gpu_huffman must be 0 ... 3");
             ctx->opt_gpu_huffman = value;
@@ -215,6 +219,7 @@ int p2p_get_option(p2p_ctx *ctx, int key, int *value) {
         case P2P_OPT_PARTIAL_UPLOAD: *value = ctx->opt_partial; return P2P_OK;
         case P2P_OPT_GPU_HUFFMAN: *value = ctx->opt_gpu_huffman; return P2P_OK;
         case P2P_OPT_HOST_WAIT: *value = ctx->opt_host_wait.load(); return P2P_OK;
+        case P2P_OPT_PNG_FORMATS: *value = ctx->opt_png_formats.load(); return P2P_OK;
         case P2P_OPT_GPU_HUFFMAN_COUNT: *value = (int)ctx->gpu_huffman_used; return P2P_OK;
 
         default: return fail(ctx, P2P_ERR_INVALID, "unknown option");

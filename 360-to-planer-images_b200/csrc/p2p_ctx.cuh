@@ -167,6 +167,7 @@ struct p2p_ctx {
     int opt_partial = 1;       // p2p_process_image transfers only the panorama rows its views can touch
     int opt_gpu_huffman = 1;   // JPEG inputs without restart markers: Huffman decoding on the device
     std::atomic<int> opt_host_wait{0};   // 1: host threads sleep while they wait for a slot's stream (see wait_slot)
+    std::atomic<int> opt_png_formats{0}; // PNG decoder subset (parse_png): 0 = 8-bit non-interlaced, 1 = every PNG format
     long long gpu_huffman_used = 0, gpu_huffman_fallback = 0;
     uint32_t *d_crc_table = nullptr;    // CRC-32 table of the PNG encoder
     p2pjpeg::Tables *d_jtab = nullptr;  // JPEG tables + header of (jW, jH, jQ): the entry of jtabs in use

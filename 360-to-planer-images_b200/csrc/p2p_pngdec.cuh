@@ -29,18 +29,24 @@
 //   6. pd_unfilter_kernel undoes the scanline filters: a warp per band of 32 rows, lane t one 4-pixel chunk behind lane
 //      t - 1 (a skewed wavefront: the reconstructed pixels above arrive through shuffles); a band whose first row needs the
 //      row above waits for the band before it (progress flags, 128 pixels at a time); rows filtered None / Sub need nothing.
-//   7. pd_bgr_kernel writes the BGR staging image (RGB / RGBA / gray / gray + alpha, 8 bit: what cv2.imread(path) with its
-//      default flag IMREAD_COLOR returns for them), which the usual pack kernel turns into the packed panorama.
+//      An Adam7 image is seven small images in a row: a launch per non-empty pass, each with its own progress flags.
+//   7. pd_bgr_kernel<colour type, bit depth, interlaced> writes the BGR staging image (what cv2.imread(path) with its default
+//      flag IMREAD_COLOR returns: gray replicated, alpha dropped, the high byte of 16-bit samples, 1/2/4-bit gray scaled,
+//      palette entries looked up), a gather that finds every pixel's Adam7 pass by its position; the usual pack kernel turns
+//      it into the packed panorama.
 //
 // Everything that touches bits (bit reader, header parser, table builder, symbol decoder, block decoder, filters) is
 // __host__ __device__ code shared with a serial host model of the same pipeline (p2p_png_decode_host, no GPU: CPU tests
 // compare it with cv2.imdecode / zlib on every kind of file before the device sees one).
 //
-// Subset: 8-bit gray / RGB / gray + alpha / RGBA, not interlaced, no APNG, no tRNS, no eXIf; anything else, any damaged file and any
+// Subset (parse_png, formats = 0, the default): 8-bit gray / RGB / gray + alpha / RGBA, not interlaced, no APNG, no PLTE, no
+// tRNS, no eXIf.  formats = 1 (P2P_OPT_PNG_FORMATS): every colour type and bit depth of the PNG specification, Adam7 too,
+// PLTE and tRNS where the specification allows them; still no APNG and no eXIf.  Anything else, any damaged file and any
 // stream whose blocks are too long to be worth it (a single huge block, fixed-Huffman-only writers) is declined
 // (P2P_ERR_UNSUPPORTED -> the caller uses cv2.imread as before).  The algorithms restated here are zlib's inflate
-// (inflate.c / inftrees.c validity rules; RFC 1951) and libpng's row filters (pngrutil.c png_read_filter_row; PNG
-// specification section 9) - see THIRD_PARTY.md.
+// (inflate.c / inftrees.c validity rules; RFC 1951), libpng's row filters (pngrutil.c png_read_filter_row; PNG
+// specification section 9) and its read transformations png_do_read_interlace, png_do_unpack / png_do_expand,
+// png_do_expand_palette and png_do_strip_16 (pngrutil.c, pngrtran.c; PNG specification sections 7, 8.2) - see THIRD_PARTY.md.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -474,15 +480,72 @@ PD_HD uint32_t unfilter_byte(uint32_t ft, uint32_t f, uint32_t a, uint32_t b, ui
     return unfilter_byte_masked(f, a, b, c, ft == 1 ? ~0u : 0u, ft == 2 ? ~0u : 0u, ft == 3 ? ~0u : 0u, ft >= 4 ? ~0u : 0u);
 }
 
-// BGR triple of one reconstructed pixel (cv2.imread(path), flag IMREAD_COLOR: gray replicated, alpha dropped)
-PD_HD void pixel_bgr(const uint8_t *px, int bpp, uint8_t *bgr) {
-    if (bpp <= 2) {
-        bgr[0] = bgr[1] = bgr[2] = px[0];
-    } else {
-        bgr[0] = px[2];
-        bgr[1] = px[1];
-        bgr[2] = px[0];
+// ---- reconstructed rows -> BGR -------------------------------------------------------------------------------------
+// Adam7 (PNG specification 8.2): pass p holds the pixels (x0 + dx i, y0 + dy j), dx = 1 << a7_sx(p), dy = 1 << a7_sy(p)
+// (one nibble per pass, pass 0 lowest)
+PD_HD int a7_x0(int p) { return (0x0102040 >> (4 * p)) & 15; }
+PD_HD int a7_y0(int p) { return (0x1020400 >> (4 * p)) & 15; }
+PD_HD int a7_sx(int p) { return (0x0112233 >> (4 * p)) & 15; }
+PD_HD int a7_sy(int p) { return (0x1122333 >> (4 * p)) & 15; }
+PD_HD int adam7_pass(int x, int y) {
+    return (y & 1) ? 6 : (x & 1) ? 5 : (y & 2) ? 4 : (x & 2) ? 3 : (y & 4) ? 2 : (x & 4) ? 1 : 0;
+}
+
+// where the conversion finds the reconstructed rows: per pass (one when not interlaced) the offset of its first row and the
+// row stride; and the palette (PLTE, RGB triples)
+struct Fmt {
+    int W, n_plte;
+    uint64_t off[7];
+    uint32_t stride[7];
+    uint8_t plte[768];
+};
+
+// the colour type / bit depth pairs the decoder handles (X(colour type, bit depth)); the first four are the default subset
+#define PD_FORMATS(X) X(0, 8) X(2, 8) X(4, 8) X(6, 8) X(0, 1) X(0, 2) X(0, 4) X(0, 16) X(2, 16) X(3, 1) X(3, 2) X(3, 4) X(3, 8) \
+    X(4, 16) X(6, 16)
+
+// BGR triple of image pixel (x, y), what cv2.imread(path) with flag IMREAD_COLOR returns: gray replicated, alpha dropped,
+// 16-bit samples cut to their high byte (libpng png_do_strip_16), 1/2/4-bit gray scaled to 8 bits and sub-byte samples
+// unpacked MSB first (png_do_unpack / png_do_expand), palette indices looked up (png_do_expand_palette), the Adam7 pass
+// found by position (png_do_read_interlace, as a gather).  false: a palette index without a PLTE entry (bgr = black).
+template <int CT, int DEPTH>
+PD_HD bool pixel_bgr(const Fmt &F, const uint8_t *recon, bool lace, int x, int y, uint8_t *bgr) {
+    int p = 0;
+    if (lace) {
+        p = adam7_pass(x, y);
+        x >>= a7_sx(p);
+        y >>= a7_sy(p);
     }
+    const uint8_t *row = recon + F.off[p] + (size_t)y * F.stride[p];
+    constexpr int CH = CT == 2 ? 3 : CT == 4 ? 2 : CT == 6 ? 4 : 1;
+    uint32_t v;
+    if (DEPTH < 8) {
+        const int bit = x * DEPTH;
+        v = ((uint32_t)row[bit >> 3] >> (8 - DEPTH - (bit & 7))) & ((1u << DEPTH) - 1u);
+        if (CT == 0) v *= 255u / ((1u << DEPTH) - 1u);
+    } else {
+        constexpr int SB = DEPTH / 8;   // bytes per sample, the most significant first
+        const uint8_t *s = row + (size_t)x * (CH * SB);
+        if (CH >= 3) {
+            bgr[0] = s[2 * SB];
+            bgr[1] = s[SB];
+            bgr[2] = s[0];
+            return true;
+        }
+        v = s[0];
+    }
+    if (CT == 3) {
+        if ((int)v >= F.n_plte) {
+            bgr[0] = bgr[1] = bgr[2] = 0;
+            return false;
+        }
+        bgr[0] = F.plte[3 * v + 2];
+        bgr[1] = F.plte[3 * v + 1];
+        bgr[2] = F.plte[3 * v];
+        return true;
+    }
+    bgr[0] = bgr[1] = bgr[2] = (uint8_t)v;
+    return true;
 }
 
 // One mark of a block's last 32 KiB during the walk through its group (block start bo, group start gs): the history byte
@@ -554,10 +617,21 @@ struct Idat {
     size_t stream_off;  // of that data in the concatenated zlib stream
     uint32_t crc;       // stored CRC (over type + data)
 };
+// a pass of an Adam7 image (a non-interlaced image is one pass: the whole image).  Its rows (filter byte + row_bytes bytes
+// each) start at raw_off of the inflated image; an empty pass (w or h = 0) has no rows at all.
+struct Pass {
+    uint32_t x0, y0, dx, dy, w, h;
+    size_t row_bytes, raw_off;
+};
 struct Info {
-    int W = 0, H = 0, color_type = 0, bpp = 0;
-    size_t row_bytes = 0;  // W * bpp
-    size_t raw_bytes = 0;  // H * (1 + row_bytes): the inflated image
+    int W = 0, H = 0, color_type = 0, bpp = 0;  // bpp: the filters' byte distance, max(1, bits per pixel / 8)
+    int depth = 8, interlace = 0;  // bits per sample; 1 = Adam7
+    size_t row_bytes = 0;  // ceil(W * bits per pixel / 8)
+    size_t raw_bytes = 0;  // sum over the passes of h * (1 + row_bytes): the inflated image
+    int n_pass = 1;
+    Pass pass[7] = {};
+    int n_plte = 0;        // palette entries (colour type 3)
+    uint8_t plte[768] = {};
     uint32_t wsize = 0;    // window of the zlib header
     size_t stream_len = 0; // bytes of the concatenated zlib stream (header and Adler-32 included)
     uint32_t adler = 0;    // stored Adler-32 (read once the end of the deflate data is known)
@@ -569,13 +643,37 @@ struct Parsed {
 
 inline uint32_t be32(const uint8_t *p) { return ((uint32_t)p[0] << 24) | ((uint32_t)p[1] << 16) | ((uint32_t)p[2] << 8) | p[3]; }
 
+// the passes of the image and the size of the inflated data (W, H, depth, interlace and bits per pixel set)
+inline void layout_passes(Info &I, int bits) {
+    I.row_bytes = ((size_t)I.W * bits + 7) / 8;
+    I.n_pass = I.interlace ? 7 : 1;
+    size_t off = 0;
+    for (int p = 0; p < I.n_pass; ++p) {
+        Pass &q = I.pass[p];
+        q.x0 = I.interlace ? a7_x0(p) : 0;
+        q.y0 = I.interlace ? a7_y0(p) : 0;
+        q.dx = I.interlace ? 1u << a7_sx(p) : 1;
+        q.dy = I.interlace ? 1u << a7_sy(p) : 1;
+        q.w = (uint32_t)I.W > q.x0 ? ((uint32_t)I.W - q.x0 + q.dx - 1) / q.dx : 0;
+        q.h = (uint32_t)I.H > q.y0 ? ((uint32_t)I.H - q.y0 + q.dy - 1) / q.dy : 0;
+        if (!q.w) q.h = 0;
+        q.row_bytes = ((size_t)q.w * bits + 7) / 8;
+        q.raw_off = off;
+        off += (size_t)q.h * (1 + q.row_bytes);
+    }
+    I.raw_bytes = off;
+}
+
 // Chunk walk.  0 = inside the subset, 1 = decline.  Checks the CRC of every chunk except IDAT (those are checked on the
 // device, or by the host model) - a file libpng rejects or merely warns about is declined.
-inline int parse_png(const uint8_t *f, size_t len, Parsed &P) {
+// formats = 0: 8-bit gray / RGB / gray + alpha / RGBA, not interlaced, no PLTE, no tRNS.  formats = 1: every colour type
+// and bit depth of the PNG specification (11.2.2), Adam7 too; PLTE and tRNS where the specification puts them (a tRNS
+// key is ignored and the palette's alpha dropped, as cv2.imread's IMREAD_COLOR does), no tRNS on types with alpha.
+inline int parse_png(const uint8_t *f, size_t len, Parsed &P, int formats = 0) {
     static const uint8_t sig[8] = {0x89, 'P', 'N', 'G', 0x0D, 0x0A, 0x1A, 0x0A};
     if (len < 8 + 25 + 12 || memcmp(f, sig, 8) != 0) return 1;
     size_t at = 8;
-    bool seen_ihdr = false, seen_idat = false, idat_closed = false, seen_iend = false;
+    bool seen_ihdr = false, seen_idat = false, idat_closed = false, seen_iend = false, seen_plte = false, seen_trns = false;
     Info &I = P.info;
     P.idat.clear();
     size_t stream_off = 0;
@@ -590,18 +688,33 @@ inline int parse_png(const uint8_t *f, size_t len, Parsed &P) {
             if (memcmp(type, "IHDR", 4) != 0 || clen != 13) return 1;
             const uint32_t W = be32(data), H = be32(data + 4);
             if (W == 0 || H == 0 || W > 0x7FFFFFFFu || H > 0x7FFFFFFFu) return 1;
-            if (data[8] != 8 || data[10] != 0 || data[11] != 0 || data[12] != 0) return 1;  // 8 bit, deflate, adaptive, not interlaced
             I.color_type = data[9];
-            I.bpp = I.color_type == 0 ? 1 : I.color_type == 2 ? 3 : I.color_type == 4 ? 2 : I.color_type == 6 ? 4 : 0;
-            if (!I.bpp) return 1;  // palette images stay with cv2
+            int bits;
+            if (!formats) {
+                if (data[8] != 8 || data[10] != 0 || data[11] != 0 || data[12] != 0) return 1;  // 8 bit, deflate, adaptive, not interlaced
+                I.bpp = I.color_type == 0 ? 1 : I.color_type == 2 ? 3 : I.color_type == 4 ? 2 : I.color_type == 6 ? 4 : 0;
+                if (!I.bpp) return 1;  // palette images stay with cv2
+                bits = 8 * I.bpp;
+            } else {
+                const int d = data[8], ct = I.color_type;
+                if (data[10] != 0 || data[11] != 0 || data[12] > 1) return 1;   // deflate, adaptive filters, none / Adam7
+                const bool ok = ct == 0 ? (d == 1 || d == 2 || d == 4 || d == 8 || d == 16)
+                                : ct == 3 ? (d == 1 || d == 2 || d == 4 || d == 8)
+                                : (ct == 2 || ct == 4 || ct == 6) && (d == 8 || d == 16);
+                if (!ok) return 1;
+                I.depth = d;
+                I.interlace = data[12];
+                bits = d * (ct == 2 ? 3 : ct == 4 ? 2 : ct == 6 ? 4 : 1);
+                I.bpp = bits < 8 ? 1 : bits / 8;
+            }
             if (W >= 32767 || H >= 32767) return 1;
             I.W = (int)W;
             I.H = (int)H;
-            I.row_bytes = (size_t)W * I.bpp;
-            I.raw_bytes = (size_t)H * (1 + I.row_bytes);
+            layout_passes(I, bits);
             seen_ihdr = true;
         } else if (is_idat) {
             if (idat_closed) return 1;  // IDAT chunks must be consecutive
+            if (I.color_type == 3 && !seen_plte) return 1;
             seen_idat = true;
             if (clen) P.idat.push_back(Idat{at + 8, clen, stream_off, stored});
             else if (crc32_host(type, 4) != stored) return 1;
@@ -614,11 +727,41 @@ inline int parse_png(const uint8_t *f, size_t len, Parsed &P) {
                 break;
             }
             if (memcmp(type, "IHDR", 4) == 0) return 1;
+            const int ct = I.color_type;
+            if (formats && memcmp(type, "PLTE", 4) == 0) {   // one, in front of IDAT; the palette of type 3, a suggestion for 2 / 6
+                if (ct == 0 || ct == 4 || seen_plte || seen_idat || clen == 0 || clen % 3 || clen > 768) return 1;
+                if (ct == 3 && (int)(clen / 3) > (1 << I.depth)) return 1;
+                if (ct == 3) {
+                    I.n_plte = (int)(clen / 3);
+                    memcpy(I.plte, data, clen);
+                }
+                seen_plte = true;
+                at += (size_t)clen + 12;
+                continue;
+            }
+            if (formats && memcmp(type, "tRNS", 4) == 0) {   // one, in front of IDAT; read by nothing here (IMREAD_COLOR)
+                if (seen_trns || seen_idat) return 1;
+                const uint32_t lim = I.depth == 16 ? 0xFFFFu : (1u << I.depth) - 1u;
+                if (ct == 0) {
+                    if (clen != 2 || ((uint32_t)data[0] << 8 | data[1]) > lim) return 1;
+                } else if (ct == 2) {
+                    if (clen != 6) return 1;
+                    for (int k = 0; k < 3; ++k)
+                        if (((uint32_t)data[2 * k] << 8 | data[2 * k + 1]) > lim) return 1;
+                } else if (ct == 3) {
+                    if (!seen_plte || clen == 0 || (int)clen > I.n_plte) return 1;
+                } else {
+                    return 1;   // types with an alpha channel have no tRNS
+                }
+                seen_trns = true;
+                at += (size_t)clen + 12;
+                continue;
+            }
             // animation, transparency key, EXIF block, and every critical chunk (PLTE, a suggested palette, included): decline
             if (memcmp(type, "acTL", 4) == 0 || memcmp(type, "fcTL", 4) == 0 || memcmp(type, "fdAT", 4) == 0 ||
                 memcmp(type, "tRNS", 4) == 0 || memcmp(type, "eXIf", 4) == 0)  // (cv2.imread rotates by the EXIF orientation)
                 return 1;
-            if (!(type[0] & 0x20)) return 1;  // critical chunk (PLTE included)
+            if (!(type[0] & 0x20)) return 1;  // critical chunk (PLTE included unless formats = 1)
             for (int k = 0; k < 4; ++k)
                 if (!((type[k] >= 'A' && type[k] <= 'Z') || (type[k] >= 'a' && type[k] <= 'z'))) return 1;
         }
@@ -743,9 +886,10 @@ inline uint32_t group_size(uint32_t n_blocks) {
 // quick -> full -> measure -> walk -> symbolic decode -> tails -> resolve -> Adler / CRC -> unfilter -> BGR, the same
 // routines in the same order, one "thread" after the other.  bgr: H rows of row_stride bytes.  0 = ok, 1 = declined.
 // stats (optional, 4 values): positions passing the quick test, candidates, blocks of the chain, blocks measured on the host.
-inline int decode_host_model(const uint8_t *f, size_t len, uint8_t *bgr, size_t row_stride, uint64_t *stats) {
+// formats: as parse_png.
+inline int decode_host_model(const uint8_t *f, size_t len, uint8_t *bgr, size_t row_stride, uint64_t *stats, int formats = 0) {
     Parsed P;
-    if (parse_png(f, len, P)) return 1;
+    if (parse_png(f, len, P, formats)) return 1;
     const Info &I = P.info;
     for (const Idat &c : P.idat) {
         uint32_t crc = crc32_host(reinterpret_cast<const uint8_t *>("IDAT"), 4);
@@ -842,21 +986,38 @@ inline int decode_host_model(const uint8_t *f, size_t len, uint8_t *bgr, size_t 
         const uint8_t *tail = reinterpret_cast<const uint8_t *>(zs) + I.stream_len - 4;
         if (((s2 << 16) | s1) != be32(tail)) return 1;
     }
-    const size_t stride = 1 + I.row_bytes;
-    for (int y = 0; y < I.H; ++y) {
-        uint8_t *row = raw.data() + (size_t)y * stride;
-        const uint8_t *up = y ? row - stride : nullptr;
-        const uint32_t ft = row[0];
-        if (ft > 4) return 1;
-        for (size_t i = 0; i < I.row_bytes; ++i) {
-            const uint32_t a = i >= (size_t)I.bpp ? row[1 + i - I.bpp] : 0, b = up ? up[1 + i] : 0,
-                           c = (up && i >= (size_t)I.bpp) ? up[1 + i - I.bpp] : 0;
-            row[1 + i] = (uint8_t)unfilter_byte(ft, row[1 + i], a, b, c);
+    Fmt F{I.W, I.n_plte, {}, {}, {}};
+    memcpy(F.plte, I.plte, sizeof(F.plte));
+    for (int p = 0; p < I.n_pass; ++p) {   // every pass filtered on its own, its first row without a row above
+        const Pass &q = I.pass[p];
+        const size_t stride = 1 + q.row_bytes;
+        F.off[p] = q.raw_off + 1;
+        F.stride[p] = (uint32_t)stride;
+        for (uint32_t y = 0; y < q.h; ++y) {
+            uint8_t *row = raw.data() + q.raw_off + (size_t)y * stride;
+            const uint8_t *up = y ? row - stride : nullptr;
+            const uint32_t ft = row[0];
+            if (ft > 4) return 1;
+            for (size_t i = 0; i < q.row_bytes; ++i) {
+                const uint32_t a = i >= (size_t)I.bpp ? row[1 + i - I.bpp] : 0, b = up ? up[1 + i] : 0,
+                               c = (up && i >= (size_t)I.bpp) ? up[1 + i - I.bpp] : 0;
+                row[1 + i] = (uint8_t)unfilter_byte(ft, row[1 + i], a, b, c);
+            }
         }
     }
-    for (int y = 0; y < I.H; ++y)
-        for (int x = 0; x < I.W; ++x) pixel_bgr(raw.data() + (size_t)y * stride + 1 + (size_t)x * I.bpp, I.bpp, bgr + (size_t)y * row_stride + 3 * (size_t)x);
-    return 0;
+    bool ok = true;
+    switch (I.color_type * 32 + I.depth) {
+#define PD_HOST_BGR(CT, D)                                                                                   \
+    case CT * 32 + D:                                                                                        \
+        for (int y = 0; y < I.H; ++y)                                                                        \
+            for (int x = 0; x < I.W; ++x)                                                                    \
+                ok &= pixel_bgr<CT, D>(F, raw.data(), I.interlace != 0, x, y, bgr + (size_t)y * row_stride + 3 * (size_t)x); \
+        break;
+        PD_FORMATS(PD_HOST_BGR)
+#undef PD_HOST_BGR
+        default: return 1;
+    }
+    return ok ? 0 : 1;
 }
 
 #ifdef __CUDACC__
@@ -1324,13 +1485,16 @@ __global__ void __launch_bounds__(256) pd_unfilter_kernel(const uint8_t *__restr
     }
 }
 
-// reconstructed rows (rstride bytes each) -> BGR staging image (row stride dstride)
-__global__ void __launch_bounds__(256) pd_bgr_kernel(const uint8_t *__restrict__ recon, int W, int H, size_t rstride, int bpp, uint8_t *__restrict__ bgr,
-                                                     size_t dstride) {
+// reconstructed rows (per pass: F.off, F.stride) -> BGR staging image (row stride dstride), a thread per image pixel
+// (grid.y = image rows).  The palette is a kernel parameter, not a __constant__ symbol: slots decode concurrently.  A palette
+// index without a PLTE entry raises *bad.
+template <int CT, int DEPTH, bool LACE>
+__global__ void __launch_bounds__(256) pd_bgr_kernel(const uint8_t *__restrict__ recon, const __grid_constant__ Fmt F, uint8_t *__restrict__ bgr,
+                                                     size_t dstride, int *bad) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
-    if (x >= W) return;
+    if (x >= F.W) return;
     uint8_t v[3];
-    pixel_bgr(recon + (size_t)y * rstride + (size_t)x * bpp, bpp, v);
+    if (!pixel_bgr<CT, DEPTH>(F, recon, LACE, x, y, v)) *bad = 1;
     uint8_t *o = bgr + (size_t)y * dstride + 3 * (size_t)x;
     o[0] = v[0];
     o[1] = v[1];

@@ -119,17 +119,19 @@ def jpeg_probe(data: bytes):
     return (w.value, h.value) if rc == 0 else None
 
 
-def png_probe(data: bytes):
-    """(W, H) if the device PNG decoder accepts this file's structure (8-bit gray / RGB / gray + alpha / RGBA, not
-    interlaced, every chunk CRC intact), else None (read it with cv2.imread).  Chunk walk only, no GPU."""
+def png_probe(data: bytes, formats: int = 0):
+    """(W, H) if the device PNG decoder accepts this file's structure (``formats`` = 0: 8-bit gray / RGB / gray + alpha /
+    RGBA, not interlaced; 1: every PNG colour type and bit depth, Adam7 too - see ``P2P_OPT_PNG_FORMATS``; every chunk CRC
+    intact), else None (read it with cv2.imread).  Chunk walk only, no GPU."""
     w, h = C.c_int(), C.c_int()
-    rc = _lib.load().p2p_png_probe(data, len(data), C.byref(w), C.byref(h))
+    rc = _lib.load().p2p_png_probe_ex(data, len(data), int(formats), C.byref(w), C.byref(h))
     return (w.value, h.value) if rc == 0 else None
 
 
-def probe_encoded(data: bytes):
-    """(W, H) if one of the device decoders handles this file (PNG by its signature, else JPEG), else None."""
-    return png_probe(data) if data[:8] == b"\x89PNG\r\n\x1a\n" else jpeg_probe(data)
+def probe_encoded(data: bytes, png_formats: int = 0):
+    """(W, H) if one of the device decoders handles this file (PNG by its signature, else JPEG), else None.
+    ``png_formats``: the PNG decoder's subset (``png_probe``)."""
+    return png_probe(data, png_formats) if data[:8] == b"\x89PNG\r\n\x1a\n" else jpeg_probe(data)
 
 
 def _as_u8_image(a, what="panorama") -> np.ndarray:
@@ -187,6 +189,7 @@ class Projector:
         for i in reversed(range(self.n_slots)):
             self._pool.put(i)
         self._lock = threading.Lock()
+        self.png_formats = 0   # P2P_OPT_PNG_FORMATS as set through set_option: the subset decode_png probes with
 
     # -- plumbing ---------------------------------------------------------------------------
     def close(self):
@@ -221,6 +224,8 @@ class Projector:
 
     def set_option(self, key: int, value: int):
         self._ck(self.lib.p2p_set_option(self.ctx, key, value))
+        if key == _lib.OPT_PNG_FORMATS:
+            self.png_formats = int(value)
 
     def get_option(self, key: int) -> int:
         v = C.c_int()
@@ -584,8 +589,9 @@ class Projector:
 
     # -- PNG panoramas decoded on the device (the decode side of cv2.imread for .png inputs, ref :244) ----------
     def png_probe(self, data: bytes):
-        """(W, H) if the device decoder accepts this file's structure, else None (read it with cv2.imread)."""
-        return png_probe(data)
+        """(W, H) if the device decoder accepts this file's structure with this context's ``P2P_OPT_PNG_FORMATS``, else
+        None (read it with cv2.imread)."""
+        return png_probe(data, self.png_formats)
 
     def upload_png(self, slot: int, data: bytes) -> tuple:
         """Decode a PNG file into ``slot`` as its panorama (inflate, unfilter and packing on the device); returns (Wp, Hp).
@@ -596,7 +602,7 @@ class Projector:
 
     def decode_png(self, data: bytes, slot: int | None = None) -> np.ndarray:
         """The array ``cv2.imdecode(data, cv2.IMREAD_COLOR)`` returns (u8 [H, W, 3], BGR), decoded on the device."""
-        dims = png_probe(data)
+        dims = png_probe(data, self.png_formats)
         if dims is None:
             raise P2PError(-6, "PNG file outside the supported subset (fall back to cv2.imread)")
         W, H = dims

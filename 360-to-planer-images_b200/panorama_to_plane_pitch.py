@@ -69,6 +69,18 @@ def set_devices(devices):
         set_device(devs[0])
 
 
+def set_png_formats(all_formats: bool):
+    """PNG inputs the device decoder takes (default False: 8-bit gray / RGB / gray + alpha / RGBA, not interlaced; True:
+    also 16-bit, palette, 1/2/4-bit gray and Adam7-interlaced files, ``P2P_OPT_PNG_FORMATS`` = 1).  Same pixels as
+    ``cv2.imread`` either way; the files left out are read with cv2.imread."""
+    global _png_formats
+    with _projectors_lock:
+        _png_formats = 1 if all_formats else 0
+        for proj in _projectors.values():
+            proj.set_option(_engine._lib.OPT_PNG_FORMATS, _png_formats)
+
+
+_png_formats = 0
 _host_checked = False
 
 
@@ -81,6 +93,8 @@ def get_projector(device: int | None = None) -> _engine.Projector:
             _engine.warn_if_host_differs(logging.getLogger())
         if d not in _projectors:
             _projectors[d] = _engine.Projector(d, n_slots=16)  # device buffers are allocated per slot on first use
+            if _png_formats:
+                _projectors[d].set_option(_engine._lib.OPT_PNG_FORMATS, _png_formats)
         return _projectors[d]
 
 
@@ -117,8 +131,9 @@ class _JpegSource:
 
 def _open_image(path):
     """``cv2.imread(path)`` of the reference (ref :244): a BGR array, or None if unreadable - except that a JPEG or PNG file
-    inside its device decoder's subset (baseline / progressive YCbCr without EXIF rotation; 8-bit non-interlaced PNG) stays as
-    bytes and is decoded on the GPU (same pixels, ``csrc/p2p_jpegdec.cuh`` / ``csrc/p2p_pngdec.cuh``)."""
+    inside its device decoder's subset (baseline / progressive YCbCr without EXIF rotation; 8-bit non-interlaced PNG, every PNG
+    format after ``set_png_formats(True)``) stays as bytes and is decoded on the GPU (same pixels, ``csrc/p2p_jpegdec.cuh`` /
+    ``csrc/p2p_pngdec.cuh``)."""
     import cv2
 
     path = Path(path)
@@ -128,7 +143,7 @@ def _open_image(path):
         except OSError:
             data = b""
         # by content, like cv2.imread (which looks at the signature, not at the suffix)
-        dims = _engine.probe_encoded(data) if data else None
+        dims = _engine.probe_encoded(data, png_formats=_png_formats) if data else None
         if dims is not None:
             return _JpegSource(data, dims, path)
     return cv2.imread(str(path))
@@ -712,6 +727,9 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--devices", type=int, nargs="+", default=None,
                    help="several CUDA devices: the files of a folder are sharded round-robin, a single image is split "
                         "by output row bands / views (extra flag)")
+    p.add_argument("--png_all_formats", action="store_true",
+                   help="decode 16-bit, palette, 1/2/4-bit gray and interlaced PNG inputs on the GPU too (extra flag; same "
+                        "pixels as cv2.imread)")
     p.add_argument("-v", "--version", action="version", version=f"%(prog)s {get_version()}",
                    help="Show version information")
     return p
@@ -726,6 +744,7 @@ def cli(argv=None):
         handlers.append(logging.FileHandler(log_file_path, mode="a"))
     logging.basicConfig(level=logging.INFO, format="%(asctime)s [%(levelname)s] %(message)s", handlers=handlers)
     set_device(args.device)
+    set_png_formats(args.png_all_formats)
     main(
         input_path=args.input_path, output_path=args.output_path, yaw_angles=args.yaw_angles,
         pitch_angles=args.pitch_angles, output_width=args.output_width, output_height=args.output_height,

@@ -89,6 +89,11 @@ typedef enum p2p_option {
                                      default spins: lowest latency, one busy core per waiting thread - the reference's
                                      ThreadPoolExecutor workers, ref :252-265, block in cv2 instead); 1: the thread sleeps on a
                                      blocking-sync event, for more images in flight than cores (several ranks on one box) */
+    ,P2P_OPT_PNG_FORMATS = 14      /* PNG files the device decoder takes (p2p_upload_pano_png, p2p_decode_png; ref :244).
+                                     0 (default): 8-bit gray / RGB / gray + alpha / RGBA, not interlaced, no PLTE, no tRNS;
+                                     1: also 1/2/4/16-bit gray, 16-bit RGB / gray + alpha / RGBA, palette images (1/2/4/8
+                                     bit) and Adam7 interlacing, tRNS on gray / RGB / palette images - with the pixels
+                                     cv2.imread's IMREAD_COLOR returns (high byte of 16-bit samples, palette alpha dropped) */
     ,P2P_OPT_SEG_CHUNKS = 11       /* row-segment kernel: chunks of 32 pixel pairs per warp (default 4, 1..64) */
     ,P2P_OPT_PARTIAL_UPLOAD = 8    /* 1 (default): p2p_process_image copies only the panorama rows its views can
                                      touch (p2p_view_row_range) over PCIe; 0: always the whole panorama */
@@ -275,12 +280,19 @@ int p2p_decode_jpeg(p2p_ctx *ctx, int slot, const uint8_t *file, size_t len, uin
  * not interlaced, no APNG, no tRNS, every chunk CRC intact), else P2P_ERR_UNSUPPORTED - the caller then reads the file
  * with cv2.imread as before. */
 int p2p_png_probe(const uint8_t *file, size_t len, int *W, int *H);
+/* p2p_png_probe for a subset: formats as P2P_OPT_PNG_FORMATS (0: p2p_png_probe; 1: every PNG colour type, bit depth and
+ * Adam7).  The same rule cv2.imread(path) of a .png input is replaced by (ref :244). */
+int p2p_png_probe_ex(const uint8_t *file, size_t len, int formats, int *W, int *H);
 /* Host model of the device decoder (no GPU, debug / tests): the same routines - block-start search, chain walk, inflate
  * with symbolic history, resolution, Adler-32 / CRC-32 checks, unfilter - run serially.  bgr: capacity_rows rows of
  * row_stride bytes, the array cv2.imread(path) returns.  stats (optional, 4 values): bit positions passing the first
  * header test, block-start candidates, deflate blocks of the stream, blocks the chain walk had to measure itself. */
 int p2p_png_decode_host(const uint8_t *file, size_t len, uint8_t *bgr, size_t row_stride, size_t capacity_rows,
                         uint64_t *stats);
+/* p2p_png_decode_host for a subset (formats as P2P_OPT_PNG_FORMATS; ref :244): also the unpacking of 1/2/4-bit samples,
+ * the palette look-up, the high byte of 16-bit samples and the Adam7 passes, by the routines the device runs. */
+int p2p_png_decode_host_ex(const uint8_t *file, size_t len, int formats, uint8_t *bgr, size_t row_stride, size_t capacity_rows,
+                           uint64_t *stats);
 /* Decode the file into `slot` as its panorama (like cv2.imread + p2p_upload_pano, identical pixels): the deflate stream is
  * inflated in parallel on the device (block starts found by testing every bit position for a dynamic-block header, every
  * block decoded independently with symbolic history, back-references resolved afterwards), the scanline filters are undone
