@@ -70,7 +70,8 @@ typedef enum p2p_option {
                                      half up); integer-roll yaws only */
     ,P2P_OPT_TRIG = 7              /* 0 (default): f32 arccos / arctan2 exactly as NumPy evaluates them on AVX-512
                                      hosts (Intel SVML, ref :162-164) - coordinates and pixels then match the
-                                     reference bit for bit there; 1: table-free minimax fits (<= 1.2 ulp) */
+                                     reference bit for bit there; 1: table-free minimax fits (acos <= 1.07 ulp,
+                                     atan2 <= 1.76 ulp, measured on a B200) */
     ,P2P_OPT_GPU_HUFFMAN = 9       /* 1 (default): JPEG inputs are Huffman-decoded on the device (self-synchronising
                                      subsequences, restart intervals as independent scans), the FF 00 stuffing of files
                                      without restart markers is removed on the device too, and the whole stage is queued

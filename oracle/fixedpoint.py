@@ -133,20 +133,22 @@ def fma32(a, b, c):
     return bits.view(np.float64).astype(np.float32)
 
 
-def pitch_coords_scalar_model(W, H, fov_deg, pitch_deg, Wp, Hp):
+def pitch_coords_scalar_model(W, H, fov_deg, pitch_deg, Wp, Hp, rows=None):
     """Per-pixel op sequence of SURVEY Appendix A steps 1-5 (what the CUDA kernel executes),
     with NumPy's own f32 ``arccos`` / ``arctan2`` for the two transcendentals.
 
     Unlike ``ref_port.pitch_mapping`` this does not call sgemm: the rotation is the explicit
     k-ordered FMA chain.  ``tests/test_oracle_golden.py`` asserts it equals the reference map
-    bit for bit on this host.
+    bit for bit on this host.  ``rows``: compute only these output rows (maps of shape
+    [len(rows), W]), for views too large to map whole.
     """
     f, c, s = ref_port.pitch_scalars(W, fov_deg, pitch_deg)
     u = np.arange(W, dtype=np.float32)[None, :]
-    v = np.arange(H, dtype=np.float32)[:, None]
-    x = np.broadcast_to(u - np.float32(W / 2.0), (H, W))
-    y = np.broadcast_to(np.float32(H / 2.0) - v, (H, W))
-    z = np.full((H, W), f, dtype=np.float32)
+    v = (np.arange(H) if rows is None else np.asarray(rows)).astype(np.float32)[:, None]
+    shape = (v.shape[0], W)
+    x = np.broadcast_to(u - np.float32(W / 2.0), shape)
+    y = np.broadcast_to(np.float32(H / 2.0) - v, shape)
+    z = np.full(shape, f, dtype=np.float32)
     n = np.sqrt((x * x + y * y) + z * z)
     xn, yn, zn = x / n, y / n, z / n
     zero = np.float32(0) * xn
@@ -180,10 +182,13 @@ def sample_view(pano, U, V, yaw_ix=None, yaw_shift=None):
     iy1 = np.clip(iy + 1, 0, Hp - 1)
     c0 = yaw_ix[ix0]
     c1 = yaw_ix[ix1]
-    p = pano.astype(np.int64)
+
+    def p(yy, xx):   # gather first: the taps, not the whole panorama, are widened to int64
+        return pano[yy, xx].astype(np.int64)
+
     wx0, wy0 = (INTER_TAB - fx)[..., None], (INTER_TAB - fy)[..., None]
     wx1, wy1 = fx[..., None], fy[..., None]
-    acc = p[iy0, c0] * wx0 * wy0 + p[iy0, c1] * wx1 * wy0 + p[iy1, c0] * wx0 * wy1 + p[iy1, c1] * wx1 * wy1
+    acc = p(iy0, c0) * wx0 * wy0 + p(iy0, c1) * wx1 * wy0 + p(iy1, c0) * wx0 * wy1 + p(iy1, c1) * wx1 * wy1
     out = ((acc + 512) >> 10).astype(np.uint8)
     out[dead] = 0
     return out

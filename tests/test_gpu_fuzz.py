@@ -32,10 +32,16 @@ def test_random_configs_against_oracle(proj, case):
     smooth = synth.smooth(Wp, Hp, Wp + H)
     got_n = proj.project_image(noise, yaws, pitches, W, H, fov)
     got_s = proj.project_image(smooth, yaws, pitches, W, H, fov)
+    # When this host's NumPy evaluates arccos / arctan2 with SVML (AVX-512), the default device path is
+    # bit-identical to the oracle; otherwise the reference itself differs in the last ulp on this host.
+    strict = svml_model.host_numpy_uses_svml()
     with proj.slots(1) as (s,):
         proj.upload(s, noise)
         for j, p in enumerate(pitches):
             U, V = ref_port.pitch_mapping(W, H, fov, p, Wp, Hp)
+            if strict:   # the default coordinates are NumPy's, bit for bit (NaN as NaN)
+                Ud, Vd = proj.coords(W, H, fov, p, Wp, Hp)
+                assert np.array_equal(Ud, U, equal_nan=True) and np.array_equal(Vd, V, equal_nan=True), (case, p)
             # sampler stage with the oracle's maps: bit-exact for every integer-roll yaw
             for y in yaws:
                 ix, fx = fp.yaw_column_table(Wp, y)
@@ -43,9 +49,6 @@ def test_random_configs_against_oracle(proj, case):
                 if shift is not None:
                     assert np.array_equal(proj.sample_with_maps(s, shift, U, V),
                                           fp.sample_view(noise, U, V, yaw_shift=shift)), (case, y, p)
-    # When this host's NumPy evaluates arccos / arctan2 with SVML (AVX-512), the default device path is
-    # bit-identical to the oracle; otherwise the reference itself differs in the last ulp on this host.
-    strict = svml_model.host_numpy_uses_svml()
     total = exact = 0
     for i, y in enumerate(yaws):
         for j, p in enumerate(pitches):

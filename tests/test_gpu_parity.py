@@ -13,13 +13,15 @@ import numpy as np
 import pytest
 
 from oracle import fixedpoint as fp
-from oracle import golden, ref_port, synth
+from oracle import golden, ref_port, svml_model, synth
 
 pytestmark = pytest.mark.gpu
 
-# G2 tolerance: |dU|, |dV| in ulps of the f32 map value.  NumPy's own arccos / arctan2 are up to
-# 2 / 3 ulp from correctly rounded (SURVEY probe p6), CUDA's are documented at 2 ulp, and the
-# final multiply / divide can move the result by one more.
+# G2 tolerance of the minimax mode: |dU|, |dV| in ulps of the f32 map value.  The reference's arctan2 /
+# arccos are up to 3 / 2 ulp off (SVML's low-accuracy variants), atan2_fast / acos_fast up to 1.76 / 1.07 ulp
+# (measured over their domains, tests/test_gpu_device_math.py).  After that, both sides round phi = a + 2 pi,
+# phi * Wp and the division by 2 pi (theta * Hp and the division by pi for V), 0.5 ulp each:
+# U: 3 + 1.76 + 2 * 1.5 = 7.76, V: 2 + 1.07 + 2 * 1.0 = 5.07, so 8 ulp bounds both.
 COORD_ULP_TOL = 8
 # G3 on noise: a coordinate within an ulp of a 1/32-px bin edge flips the bin (about 1 % of
 # pixels at 8K, SURVEY probe p4); everything else must be identical.
@@ -42,6 +44,16 @@ def ulp_diff(a, b):
 
 def exact_fraction(a, b):
     return float((a == b).all(axis=-1).mean())
+
+
+def assert_noise_view(got, want, floor, *info):
+    """Default (NumPy-exact) trig on noise: identical wherever this host's NumPy evaluates arccos / arctan2 with
+    SVML (the routines the kernels restate); elsewhere the reference itself moves in the last ulp, so only the
+    exact-pixel fraction is bounded."""
+    if svml_model.host_numpy_uses_svml():
+        assert np.array_equal(got, want), (exact_fraction(got, want), *info)
+    else:
+        assert exact_fraction(got, want) >= floor, (exact_fraction(got, want), *info)
 
 
 # ------------------------------------------------------------------------------------------
@@ -303,7 +315,7 @@ def test_fractional_yaw_rotate_bit_exact_and_end_to_end(proj, golden_dir):
     out = proj.project_image(pano, [int(y) for y in g["yaws"]], [int(p) for p in g["pitches"]], W, H, fov)
     for i in range(len(g["yaws"])):
         for j in range(len(g["pitches"])):
-            assert exact_fraction(out[i, j], g["out"][i, j]) >= NOISE_EXACT_MIN
+            assert_noise_view(out[i, j], g["out"][i, j], NOISE_EXACT_MIN, i, j)
 
 
 def test_fractional_yaw_one_pass_equals_the_two_passes(pkg, proj):
@@ -421,7 +433,7 @@ def test_mirror_kernel_against_per_pixel_kernel_and_oracle(pkg, proj):
         for i, y in enumerate(yaws):
             for j, p in enumerate(pitches):
                 want = fp.project_view_single_pass(noise, y, p, W, H, fov)
-                assert exact_fraction(got_n[i, j], want) >= NOISE_EXACT_MIN, (Wp, W, y, p)
+                assert_noise_view(got_n[i, j], want, NOISE_EXACT_MIN, Wp, W, y, p)
                 want_s = fp.project_view_single_pass(smooth, y, p, W, H, fov)
                 assert np.abs(got_s[i, j].astype(np.int16) - want_s.astype(np.int16)).max() <= 1, (Wp, W, y, p)
 
@@ -462,7 +474,7 @@ def test_exact_bilinear_mode_against_scipy(pkg):
                     if kind == "smooth":
                         assert np.abs(out[i, j].astype(np.int16) - want.astype(np.int16)).max() <= 1
                     else:
-                        assert exact_fraction(out[i, j], want) >= 0.97
+                        assert_noise_view(out[i, j], want, 0.97, y, pt)
         with pytest.raises(pkg.P2PError):   # fractional yaws are only defined for the cv2 mode
             p.project_image(pano, [30], [90], W, H, fov)
         # seam-wrap option: U runs over [0, Wp), pixels between the last and the first column blend the two
@@ -492,7 +504,7 @@ def test_exact_bilinear_mode_against_scipy(pkg):
                         if kind == "smooth":
                             assert np.abs(out[i, j].astype(np.int16) - want.astype(np.int16)).max() <= 1, (seam, yw, pt)
                         else:
-                            assert exact_fraction(out[i, j], want) >= 0.97, (seam, yw, pt)
+                            assert_noise_view(out[i, j], want, 0.97, seam, yw, pt)
                 clamp_views[seam] = out.copy()
         assert not np.array_equal(clamp_views[0], clamp_views[1])   # the seam column really is interpolated differently
         # and the default mode is untouched: it differs from the exact mode (5-bit fractions) on noise
@@ -616,9 +628,8 @@ def test_full_size_c4_16k(proj):
     pano = synth.noise(Wp, Hp, 0)
     out = proj.project_image(pano, [0, 90, 180, 270], [30, 60, 90], W, H, fov)
     want = fp.project_view_single_pass(pano, 90, 60, W, H, fov)
-    fr = exact_fraction(out[1, 1], want)
-    print("G3 C4 16K yaw 90 pitch 60 exact-pixel fraction", fr)
-    assert fr >= 0.93  # an ulp of U is twice as many 1/32-px bins at 16K
+    print("G3 C4 16K yaw 90 pitch 60 exact-pixel fraction", exact_fraction(out[1, 1], want))
+    assert_noise_view(out[1, 1], want, 0.93)  # without SVML: an ulp of U is twice as many 1/32-px bins at 16K
     rolled = np.roll(pano, -Wp // 2, axis=1)
     assert np.array_equal(proj.project_image(rolled, [0], [30], W, H, fov)[0, 0], out[2, 0])
 
