@@ -63,6 +63,7 @@ SIGNATURES = {
     "p2p_process_image_png": (_i, [_vp, _i, _u8p, _i, _i, _sz, _i, _i32p, _i, _pcp, _i, _i, _u8p, _sz, C.POINTER(_sz), _u8p]),
     "p2p_jpeg_probe": (_i, [_u8p, _sz, C.POINTER(_i), C.POINTER(_i)]),
     "p2p_jpeg_coefficients": (_i, [_u8p, _sz, _vp, _sz, _i32p]),
+    "p2p_jpeg_device_tables": (_i, [_u8p, _sz, _vp, _sz, _i32p]),
     "p2p_upload_pano_jpeg": (_i, [_vp, _i, _u8p, _sz, C.POINTER(_i), C.POINTER(_i)]),
     "p2p_decode_jpeg": (_i, [_vp, _i, _u8p, _sz, _u8p, _sz, _sz]),
     "p2p_png_probe": (_i, [_u8p, _sz, C.POINTER(_i), C.POINTER(_i)]),

@@ -12,6 +12,9 @@
 //                     chroma plane is at most 2 samples wide), jdcolor.c ycc_rgb_convert   (jpegdec_color_kernel)
 // Supported: 8-bit, 3 components (YCbCr; 4:4:4 / 4:2:2 / 4:2:0) or 1 (grayscale); SOF0 / SOF1 with one scan and restart
 // markers (Huffman stage on the device), SOF2 progressive files (jdphuff.c restated on the host, decode_progressive).
+// Any legal Huffman tables, not only the Annex K ones cv2 writes by default: optimised tables, codes of 9 / 10 / 16 bits,
+// AC codes whose length + size sits on the 10-bit combined look-up's edge, DC tables of up to 256 entries, size-0 symbols
+// other than 0x00 as end of block, table ids 0-3 (tests/jpeg_writer.py writes such files for the tests).
 // Anything else (CMYK, RGB-coded files, EXIF orientation != 1, damaged data) is reported as
 // unsupported and the caller falls back to cv2.imread, as the reference does for every file.
 #pragma once
@@ -673,6 +676,7 @@ inline int decode_scan(const uint8_t *d, size_t len, const Parsed &P, int16_t *c
                     br.n = 0;
                     br.marker = false;
                     br.zero_bits = 0;
+                    while (br.p + 2 <= br.end && br.p[0] == 0xFF && br.p[1] == 0xFF) ++br.p;   // fill bytes (jdmarker.c next_marker)
                     if (br.p + 2 > br.end || br.p[0] != 0xFF || br.p[1] != 0xD0 + next_rst) return 1;
                     next_rst = (next_rst + 1) & 7;
                     br.p += 2;
@@ -755,14 +759,18 @@ constexpr int kSubBits = 1024;
 constexpr int kMaxSyncRounds = 192;
 constexpr int kRoundsPerCheck = 4;   // synchronisation rounds enqueued per host-side convergence check
 
+// Symbol lists hold up to 256 entries for DC tables too: libjpeg takes any DHT of <= 256 values, a DC table only has to keep
+// every value <= 15 (jdhuff.c jpeg_make_d_derived_tbl), so a DC code of 10 bits or more may sit at index 16 or higher.
+constexpr int kHuffVals = 256;
+
 struct DevHuff {                 // one per component: its DC and AC table
     uint16_t dc_look[512];
     int32_t dc_maxcode[18], dc_valoff[18];
-    uint8_t dc_vals[16];
+    uint8_t dc_vals[kHuffVals];
     int32_t ac_fast[1 << kFastBits];
     uint16_t ac_look[512];
     int32_t ac_maxcode[18], ac_valoff[18];
-    uint8_t ac_vals[256];
+    uint8_t ac_vals[kHuffVals];
 };
 
 // Synchronisation rounds only need to know, per code word, how many bits it consumes (code + value bits) and how far it
@@ -780,7 +788,7 @@ struct SyncLut {
 
 inline void build_sync_lut(const HuffTable &dc, const HuffTable &ac, uint16_t *dc_out, uint16_t *ac_out, uint32_t *dc_w,
                            uint32_t *ac_w) {
-    auto symbol = [](const HuffTable &t, int win10, int mask, int &len) -> int {
+    auto symbol = [](const HuffTable &t, int win10, int &len) -> int {
         const uint16_t e = t.look[win10 >> (kFastBits - 9)];
         if (e) {
             len = e >> 8;
@@ -788,13 +796,13 @@ inline void build_sync_lut(const HuffTable &dc, const HuffTable &ac, uint16_t *d
         }
         if (win10 <= t.maxcode[10]) {   // jdhuff.c: the first length whose largest code is not below the prefix
             len = 10;
-            return t.vals[(win10 + t.valoff[10]) & mask];
+            return t.vals[(win10 + t.valoff[10]) & (kHuffVals - 1)];
         }
         return -1;
     };
     for (int i = 0; i < (1 << kFastBits); ++i) {
         int len = 0;
-        int s = symbol(dc, i, 15, len);
+        int s = symbol(dc, i, len);
         if (s >= 0) {
             s = (s > 15) ? 15 : s;
             dc_out[i] = (uint16_t)((len + s) | (1 << 5));
@@ -803,7 +811,7 @@ inline void build_sync_lut(const HuffTable &dc, const HuffTable &ac, uint16_t *d
             dc_out[i] = 0;
             dc_w[i] = 0;
         }
-        const int rs = symbol(ac, i, 255, len);
+        const int rs = symbol(ac, i, len);
         if (rs >= 0) {
             const int r = rs >> 4, sz = rs & 15;
             const int adv = sz ? r + 1 : (r == 15 ? 16 : 64);
@@ -813,6 +821,31 @@ inline void build_sync_lut(const HuffTable &dc, const HuffTable &ac, uint16_t *d
             ac_out[i] = 0;
             ac_w[i] = 0;
         }
+    }
+}
+
+// Everything the device Huffman stage reads of the file's tables, uploaded as one block: the three per-component tables, then
+// the unified look-up of the synchronisation rounds and the write pass.  (p2p_jpeg_device_tables exports the same bytes.)
+struct DevTables {
+    DevHuff T[3];
+    SyncLut L;
+};
+
+inline void build_device_tables(const Parsed &P, DevTables &DT) {
+    memset(&DT, 0, sizeof(DT));
+    for (int c = 0; c < 3; ++c) build_sync_lut(P.dc[P.td[c]], P.ac[P.ta[c]], DT.L.e[c][0], DT.L.e[c][1], DT.L.w[c][0], DT.L.w[c][1]);
+    for (int c = 0; c < 3; ++c) {
+        const HuffTable &d = P.dc[P.td[c]], &a = P.ac[P.ta[c]];
+        DevHuff &T = DT.T[c];
+        memcpy(T.dc_look, d.look, sizeof(d.look));
+        memcpy(T.dc_maxcode, d.maxcode, sizeof(d.maxcode));
+        memcpy(T.dc_valoff, d.valoff, sizeof(d.valoff));
+        memcpy(T.dc_vals, d.vals, sizeof(T.dc_vals));
+        memcpy(T.ac_fast, a.fast_ac, sizeof(a.fast_ac));
+        memcpy(T.ac_look, a.look, sizeof(a.look));
+        memcpy(T.ac_maxcode, a.maxcode, sizeof(a.maxcode));
+        memcpy(T.ac_valoff, a.valoff, sizeof(a.valoff));
+        memcpy(T.ac_vals, a.vals, sizeof(T.ac_vals));
     }
 }
 
@@ -854,13 +887,13 @@ __device__ __forceinline__ int extend_bits(uint32_t v, int s) {   // jdhuff.c HU
 // symbol and code length for the code at the top of `win`; -1 = no such code (garbage decoding or damaged data):
 // it consumes 16 bits
 __device__ __forceinline__ int slow_symbol(uint32_t win, const int32_t *maxcode, const int32_t *valoff,
-                                           const uint8_t *vals, int nvals_mask, int &len) {
+                                           const uint8_t *vals, int &len) {
     const uint32_t w16 = win >> 16;
     for (int l = 10; l <= 16; ++l) {
         const int32_t code = (int32_t)(w16 >> (16 - l));
         if (code <= maxcode[l]) {
             len = l;
-            return vals[(code + valoff[l]) & nvals_mask];
+            return vals[(code + valoff[l]) & (kHuffVals - 1)];
         }
     }
     len = 16;
@@ -915,7 +948,7 @@ __device__ __forceinline__ uint32_t huff_decode_range(const uint32_t *__restrict
                 len = e >> 8;
                 s = e & 0xFF;
             } else {
-                s = slow_symbol(win, H.dc_maxcode, H.dc_valoff, H.dc_vals, 15, len);
+                s = slow_symbol(win, H.dc_maxcode, H.dc_valoff, H.dc_vals, len);
             }
             if (WRITE && (s < 0 || s > 11)) damaged = true;
             s = (s < 0) ? 0 : (s > 15) ? 15 : s;
@@ -944,7 +977,7 @@ __device__ __forceinline__ uint32_t huff_decode_range(const uint32_t *__restrict
                 len = e >> 8;
                 rs = e & 0xFF;
             } else {
-                rs = slow_symbol(win, H.ac_maxcode, H.ac_valoff, H.ac_vals, 255, len);
+                rs = slow_symbol(win, H.ac_maxcode, H.ac_valoff, H.ac_vals, len);
                 if (rs < 0) {
                     if (WRITE) damaged = true;
                     rs = 0;
@@ -1157,12 +1190,12 @@ huff_sync_fast_kernel(const uint32_t *__restrict__ w, const DevHuff *__restrict_
             const DevHuff &H = T[comp];
             int len;
             if (st.z == 0) {
-                int s = slow_symbol(win, H.dc_maxcode, H.dc_valoff, H.dc_vals, 15, len);
+                int s = slow_symbol(win, H.dc_maxcode, H.dc_valoff, H.dc_vals, len);
                 s = (s < 0) ? 0 : (s > 15) ? 15 : s;
                 st.pos += (uint32_t)(len + s);
                 st.z = 1;
             } else {
-                int rs = slow_symbol(win, H.ac_maxcode, H.ac_valoff, H.ac_vals, 255, len);
+                int rs = slow_symbol(win, H.ac_maxcode, H.ac_valoff, H.ac_vals, len);
                 rs = (rs < 0) ? 0 : rs;
                 const int r = rs >> 4, s = rs & 15;
                 st.z += s ? r + 1 : (r == 15 ? 16 : 64);
@@ -1297,14 +1330,14 @@ huff_write_fast_kernel(const uint32_t *__restrict__ w, const DevHuff *__restrict
             const DevHuff &H = T[comp];
             int len;
             if (st.z == 0) {
-                int s = slow_symbol(win, H.dc_maxcode, H.dc_valoff, H.dc_vals, 15, len);
+                int s = slow_symbol(win, H.dc_maxcode, H.dc_valoff, H.dc_vals, len);
                 if (s < 0 || s > 11) damaged = true;
                 s = (s < 0) ? 0 : (s > 15) ? 15 : s;
                 dcdiff[(size_t)comp * G.dc_stride + dc_idx] = s ? extend_bits((win << len) >> (32 - s), s) : 0;
                 st.pos += (uint32_t)(len + s);
                 st.z = 1;
             } else {
-                int rs = slow_symbol(win, H.ac_maxcode, H.ac_valoff, H.ac_vals, 255, len);
+                int rs = slow_symbol(win, H.ac_maxcode, H.ac_valoff, H.ac_vals, len);
                 if (rs < 0) {
                     damaged = true;
                     rs = 0;

@@ -261,6 +261,12 @@ int p2p_jpeg_probe(const uint8_t *file, size_t len, int *W, int *H);
  * if coef != NULL the quantised coefficients (int16, natural order, component planes [by][bx][64], Y then Cb then Cr;
  * capacity in elements) exactly as jdhuff.c decodes them. */
 int p2p_jpeg_coefficients(const uint8_t *file, size_t len, int16_t *coef, size_t capacity, int32_t *layout);
+/* Host only (no GPU, debug / tests): the Huffman tables the device stage uploads for a baseline file, byte for byte (the
+ * DevTables block of csrc/p2p_jpegdec.cuh: per component DevHuff, then SyncLut), into out[capacity] if out != NULL;
+ * layout[16] = {sizeof DevTables, sizeof DevHuff, offsets in DevHuff of dc_look, dc_maxcode, dc_valoff, dc_vals, ac_fast,
+ * ac_look, ac_maxcode, ac_valoff, ac_vals, entries of dc_vals, of ac_vals, offset of SyncLut, offset of SyncLut.w,
+ * lookahead bits of ac_fast / SyncLut}.  P2P_ERR_UNSUPPORTED for files outside the subset and progressive files. */
+int p2p_jpeg_device_tables(const uint8_t *file, size_t len, uint8_t *out, size_t capacity, int32_t *layout);
 /* Decode the file into `slot` as its panorama (like cv2.imread + p2p_upload_pano, bit-identical pixels): Huffman
  * decoding (self-synchronising subsequences; P2P_OPT_GPU_HUFFMAN), inverse DCT, chroma upsampling and colour
  * conversion all run on the device (the FF 00 byte stuffing is removed there too when the file has no restart markers); the

@@ -10,9 +10,11 @@ from tools import synth_inputs as synth
 SAMPLING = [cv2.IMWRITE_JPEG_SAMPLING_FACTOR_420, cv2.IMWRITE_JPEG_SAMPLING_FACTOR_422, cv2.IMWRITE_JPEG_SAMPLING_FACTOR_444]
 
 
-def damaged_files(seed: int, count: int, max_wh=(120, 90), gray_every: int = 0, progressive_every: int = 0):
+def damaged_files(seed: int, count: int, max_wh=(120, 90), gray_every: int = 0, progressive_every: int = 0, writer=None):
     """Yields (label, bytes).  ``gray_every`` = k: every k-th file is a grayscale JPEG; ``progressive_every`` = k: every
-    k-th file (offset by one) is a progressive JPEG."""
+    k-th file (offset by one) is a progressive JPEG.  ``writer``: None = cv2's default (Annex K) tables, "optimize" = cv2's
+    IMWRITE_JPEG_OPTIMIZE tables, or a tests/jpeg_writer.py table policy (the cv2 file re-encoded with it before the
+    damage; no progressive files then)."""
     rng = np.random.default_rng(seed)
     for i in range(count):
         w, h = int(rng.integers(16, max_wh[0])), int(rng.integers(16, max_wh[1]))
@@ -22,9 +24,16 @@ def damaged_files(seed: int, count: int, max_wh=(120, 90), gray_every: int = 0, 
         rst, q = int(rng.integers(0, 4)), int(rng.integers(5, 100))
         samp = SAMPLING[int(rng.integers(0, 3))]
         prog = 1 if progressive_every and i % progressive_every == (1 if progressive_every > 1 else 0) else 0
-        data = bytearray(cv2.imencode(".jpg", img, [cv2.IMWRITE_JPEG_QUALITY, q, cv2.IMWRITE_JPEG_RST_INTERVAL, rst,
-                                                    cv2.IMWRITE_JPEG_SAMPLING_FACTOR, samp,
-                                                    cv2.IMWRITE_JPEG_PROGRESSIVE, prog])[1].tobytes())
+        if writer not in (None, "optimize"):
+            prog = 0
+        data = cv2.imencode(".jpg", img, [cv2.IMWRITE_JPEG_QUALITY, q, cv2.IMWRITE_JPEG_RST_INTERVAL, rst,
+                                          cv2.IMWRITE_JPEG_SAMPLING_FACTOR, samp, cv2.IMWRITE_JPEG_PROGRESSIVE, prog,
+                                          cv2.IMWRITE_JPEG_OPTIMIZE, int(writer == "optimize")])[1].tobytes()
+        if writer not in (None, "optimize"):
+            import jpeg_writer
+
+            data = jpeg_writer.write(data, tables=writer)
+        data = bytearray(data)
         sos = data.find(b"\xff\xda")
         lo, hi = ((2, sos + 14), (sos + 14, len(data) - 2), (2, len(data) - 2))[int(rng.integers(0, 3))]
         mode = int(rng.integers(0, 3))
@@ -37,7 +46,7 @@ def damaged_files(seed: int, count: int, max_wh=(120, 90), gray_every: int = 0, 
             del data[int(rng.integers(lo, hi))]
         else:
             data.insert(int(rng.integers(lo, hi)), int(rng.integers(0, 256)))
-        yield f"{i}:{w}x{h} q{q} rst{rst} mode{mode}{' progressive' if prog else ''} [{lo},{hi})", bytes(data)
+        yield f"{i}:{w}x{h} q{q} rst{rst} mode{mode}{' progressive' if prog else ''}{' ' + writer if writer else ''} [{lo},{hi})", bytes(data)
 
 
 def colour_space_variants(img):

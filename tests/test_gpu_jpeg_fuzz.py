@@ -64,30 +64,32 @@ def test_largest_shapes(proj):
 def test_damaged_files_are_declined_or_decode_like_cv2(pkg, proj, capfd):
     """tests/jpeg_damage.py through the whole device decoder, with the Huffman stage on the device and on the host: a
     damaged file is declined (-6: the front end then uses cv2.imread, like the reference) or decodes to cv2's pixels;
-    a file cv2 cannot read is always declined.  Larger images than the CPU test so that scans span many subsequences."""
+    a file cv2 cannot read is always declined.  Larger images than the CPU test so that scans span many subsequences;
+    files with cv2's default and with its optimised Huffman tables."""
     from jpeg_damage import damaged_files
 
     L = pkg._lib
     counts = {}
-    for device_stage in (1, 0):
-        proj.set_option(L.OPT_GPU_HUFFMAN, device_stage)
-        declined = same = 0
-        try:
-            for label, data in damaged_files(77, 300, max_wh=(400, 300), gray_every=5, progressive_every=4):
-                ref = cv2.imdecode(np.frombuffer(data, np.uint8), cv2.IMREAD_COLOR)
-                try:
-                    got = proj.decode_jpeg(data)
-                except pkg.P2PError as e:
-                    assert e.code == -6, (label, e)
-                    declined += 1
-                    continue
-                assert ref is not None, label
-                assert np.array_equal(got, ref), (label, device_stage)
-                same += 1
-        finally:
-            proj.set_option(L.OPT_GPU_HUFFMAN, 1)
-        counts[device_stage] = (declined, same)
-        assert declined > 30 and same > 30, counts
+    for writer, seed, n in ((None, 77, 300), ("optimize", 78, 150)):
+        for device_stage in (1, 0):
+            proj.set_option(L.OPT_GPU_HUFFMAN, device_stage)
+            declined = same = 0
+            try:
+                for label, data in damaged_files(seed, n, max_wh=(400, 300), gray_every=5, progressive_every=4, writer=writer):
+                    ref = cv2.imdecode(np.frombuffer(data, np.uint8), cv2.IMREAD_COLOR)
+                    try:
+                        got = proj.decode_jpeg(data)
+                    except pkg.P2PError as e:
+                        assert e.code == -6, (label, e)
+                        declined += 1
+                        continue
+                    assert ref is not None, label
+                    assert np.array_equal(got, ref), (label, device_stage)
+                    same += 1
+            finally:
+                proj.set_option(L.OPT_GPU_HUFFMAN, 1)
+            counts[(writer, device_stage)] = (declined, same)
+            assert declined > n // 10 and same > n // 10, counts
     capfd.readouterr()
     # the decoder still works after all that
     img = synth.smooth(320, 200, 3)

@@ -210,19 +210,24 @@ def test_damaged_files_are_declined_or_decode_like_cv2(pkg, capfd):
     from oracle import jpeg_decode_model as jd
 
     lib = pkg._lib.load()
-    declined = same = 0
-    for label, data in damaged_files(2025, 400, gray_every=4, progressive_every=3):
-        ref = cv2.imdecode(np.frombuffer(data, np.uint8), cv2.IMREAD_COLOR)
-        st, planes = _host_stage(lib, data)
-        if st:
-            assert st == -6, label
-            declined += 1
-            continue
-        assert ref is not None, label
-        assert np.array_equal(jd.reconstruct(jd.parse(data), planes), ref), label
-        same += 1
+    # cv2's default tables, its optimised tables, and hand-built ones (16-bit codes only, a DC table of 28 entries whose
+    # codes in use sit at index 16 and up, size-0 symbols other than 0x00 as end of block)
+    for writer, seed, n in ((None, 2025, 400), ("optimize", 2026, 160), ("all_len(16)", 2027, 60), ("dc_dup", 2028, 60),
+                            ("eob_alias", 2029, 60)):
+        declined = same = 0
+        for label, data in damaged_files(seed, n, gray_every=4, progressive_every=3, writer=writer):
+            ref = cv2.imdecode(np.frombuffer(data, np.uint8), cv2.IMREAD_COLOR)
+            st, planes = _host_stage(lib, data)
+            if st:
+                assert st == -6, label
+                declined += 1
+                continue
+            assert ref is not None, label
+            assert np.array_equal(jd.reconstruct(jd.parse(data), planes), ref), label
+            same += 1
+        # (damage in 16-bit codes mostly makes codes that do not exist: few of those files stay decodable)
+        assert declined > n // 8 and same > (50 if writer is None else 3), (writer, declined, same)
     capfd.readouterr()               # libjpeg's warnings about the damaged files
-    assert declined > 50 and same > 50
 
 
 def test_known_damage_patterns_are_declined(pkg):
@@ -264,8 +269,10 @@ def test_known_damage_patterns_are_declined(pkg):
 
 
 def test_host_decoder_under_address_sanitizer(tmp_path):
-    """The header parser and the host Huffman decoder, built with ASan + UBSan (tools/asan_jpeg_host.cu), on seeded
-    damaged files incl. garbage runs and truncations: no out-of-bounds access, no undefined behaviour."""
+    """The header parser, the device table builder and the host Huffman decoder, built with ASan + UBSan
+    (tools/asan_jpeg_host.cu), on seeded damaged files incl. garbage runs and truncations, with cv2's default, optimised and
+    hand-built tables: no out-of-bounds access, no undefined behaviour."""
+    import itertools
     import shutil
     import subprocess
     from pathlib import Path
@@ -283,7 +290,12 @@ def test_host_decoder_under_address_sanitizer(tmp_path):
         pytest.skip("sanitizer runtime not available: " + build.stderr[-300:])
     rng = np.random.default_rng(9)
     names = []
-    for k, (label, data) in enumerate(damaged_files(301, 600, gray_every=3, progressive_every=4)):
+    files = itertools.chain(damaged_files(301, 600, gray_every=3, progressive_every=4),
+                            damaged_files(302, 150, gray_every=3, progressive_every=4, writer="optimize"),
+                            damaged_files(303, 60, gray_every=3, writer="all_len(16)"),
+                            damaged_files(304, 60, gray_every=3, writer="dc_dup"),
+                            damaged_files(305, 60, gray_every=3, writer="fast_ac_edge"))
+    for k, (label, data) in enumerate(files):
         d = bytearray(data)
         if k % 3 == 0:                                     # heavier damage: garbage runs, truncation
             for _ in range(int(rng.integers(1, 6))):

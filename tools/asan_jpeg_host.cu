@@ -1,5 +1,5 @@
-// AddressSanitizer / UBSan harness for the HOST half of the JPEG decoder (header parser + Huffman decoder of
-// csrc/p2p_jpegdec.cuh): every file named on the command line is read into an exact-size heap buffer and decoded.
+// AddressSanitizer / UBSan harness for the HOST half of the JPEG decoder (header parser, device table builder and Huffman
+// decoder of csrc/p2p_jpegdec.cuh): every file named on the command line is read into an exact-size heap buffer and decoded.
 // No CUDA call is made, so it runs without a GPU.
 //   nvcc -O1 -g -Xcompiler -fsanitize=address,-fsanitize=undefined,-fno-omit-frame-pointer \
 //        -gencode arch=compute_100a,code=sm_100a -o /tmp/asan_jpeg_host tools/asan_jpeg_host.cu -lasan -lubsan
@@ -24,6 +24,10 @@ int main(int argc, char **argv) {
         fclose(f);
         p2pjdec::Parsed P;
         if (p2pjdec::parse_headers(buf, (size_t)n, P) == 0) {
+            if (!P.progressive) {   // the tables the device stage would upload
+                std::vector<unsigned char> mem(sizeof(p2pjdec::DevTables));
+                p2pjdec::build_device_tables(P, *reinterpret_cast<p2pjdec::DevTables *>(mem.data()));
+            }
             std::vector<int16_t> coef(P.info.n_coef);
             if (p2pjdec::decode_scan(buf, (size_t)n, P, coef.data()) == 0) ++decoded;
             else ++declined;
