@@ -83,6 +83,11 @@ void p2p_destroy(p2p_ctx *ctx) {
         if (s.tex) cudaDestroyTextureObject(s.tex);
         if (s.surf) cudaDestroySurfaceObject(s.surf);
         if (s.arr) cudaFreeArray(s.arr);
+        for (int c = 0; c < 3; ++c) {
+            if (s.ftex[c]) cudaDestroyTextureObject(s.ftex[c]);
+            if (s.fsurf[c]) cudaDestroySurfaceObject(s.fsurf[c]);
+            if (s.farr[c]) cudaFreeArray(s.farr[c]);
+        }
         cudaFree(s.d_bgr);
         cudaFree(s.d_rgba);
         cudaFree(s.d_out);

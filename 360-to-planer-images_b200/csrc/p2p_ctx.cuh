@@ -50,6 +50,17 @@ struct Slot {
     cudaTextureObject_t tex = 0;
     cudaSurfaceObject_t surf = 0;  // the same array, written directly by the pack kernel
     bool tex_current = false;
+    // yaw-folded planes (B, G, R) of the quarter-turn sampler, allocated when a panorama renders a quarter-turn group for
+    // the second time: (Wp / 4 + 1) x Hp u32 texels each, see fold_kernel
+    cudaArray_t farr[3] = {nullptr, nullptr, nullptr};
+    int farrW = 0, farrH = 0;
+    cudaTextureObject_t ftex[3] = {0, 0, 0};
+    cudaSurfaceObject_t fsurf[3] = {0, 0, 0};
+    bool fold_current = false;  // the planes hold the panorama of d_rgba (every writer of d_rgba clears it)
+    // The panorama of d_rgba has rendered a quarter-turn group from the RGBA texture: the next such launch folds it.  On a
+    // B200 the fold costs about one 12-view render (8K: 47 us) and saves ~3 % of every later one, so a panorama rendered
+    // once (the files flow, p2p_process_image) never pays it; a resident panorama rendered again and again does.
+    bool quarter_seen = false;
     uint8_t *d_out = nullptr;  // device outputs when the caller wants them on the host
     size_t out_cap = 0;
     int32_t *d_tab = nullptr;  // yaw table (ix | fx), 2 * Wp
@@ -269,6 +280,8 @@ int prepare_slot(p2p_ctx *ctx, Slot &s, int Wp, int Hp) {
     s.Hp = Hp;
     s.pitch_tex = pitch_tex;
     s.tex_current = false;
+    s.fold_current = false;
+    s.quarter_seen = false;
     return P2P_OK;
 }
 

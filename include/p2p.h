@@ -56,7 +56,8 @@ typedef enum p2p_option {
     P2P_OPT_SAMPLER = 0, /* 0 = global-load gather, 1 = texture gather4 point fetch (default) */
     P2P_OPT_WARP_W = 1,  /* output pixels per warp row: 32 (default) or 8 (8 x 4 warp tiles) */
     P2P_OPT_YAWS_PER_THREAD = 2, /* 1..4 views sharing one coordinate evaluation (default 4) */
-    P2P_OPT_COUNT_LAUNCHES = 3,  /* read-only via p2p_get_option: kernels launched so far */
+    P2P_OPT_COUNT_LAUNCHES = 3,  /* read-only via p2p_get_option: kernels launched so far (the fold of a panorama into
+                                    its quarter-turn planes, like the refresh of its texture array, is not counted) */
     P2P_OPT_IMAGES_PER_LAUNCH = 4, /* 1 (default), 2 or 4 resident panoramas share one launch (and one
                                      coordinate evaluation) in p2p_project_batch */
     P2P_OPT_MIRROR = 5            /* with the texture sampler and W % 8 == 0 the pixel pair (W/2 + t, W/2 - t) shares
@@ -172,7 +173,10 @@ int p2p_project_batch(p2p_ctx *ctx, int n_images, const int32_t *slots, int n_ya
  * unit the reference parallelises over (one (yaw, pitch) pair of the nested loops at ref :202-219 / :253-265) without the
  * yaw x pitch product structure of p2p_project_views: the six cube faces of BASELINE configs[4] - four yaws at pitch 90
  * plus the two pole pitches - are one call and one kernel launch.  Views whose pitch constants are bit-identical share one
- * coordinate evaluation (the reference's pitch_mapping_cache key has no yaw, ref :55-73).  The row band is how one image
+ * coordinate evaluation (the reference's pitch_mapping_cache key has no yaw, ref :55-73); four of them whose rolls are
+ * quarter turns apart (r0 + k Wp / 4, Wp % 4 == 0) are read automatically from the slot's yaw-folded copy, 3 texture
+ * gathers per pixel for the four views instead of 4, from the second such render of a panorama on (the fold is built
+ * then, once per panorama, and not counted in P2P_OPT_COUNT_LAUNCHES).  The row band is how one image
  * is split over several GPUs (SURVEY 8e): every device renders rows [H r / n, H (r + 1) / n) of all views into the same
  * host array.  out_on_device as in p2p_project_views (a host `out` receives only the band, one strided copy). */
 int p2p_project_view_list(p2p_ctx *ctx, int slot, int n_views, const int32_t *yaw_shift, const p2p_pitch_consts *pitch,
