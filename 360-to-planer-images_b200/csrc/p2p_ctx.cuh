@@ -83,7 +83,7 @@ struct Slot {
     size_t pg_F_cap = 0;
     uint16_t *pg_tlen = nullptr;
     size_t pg_tlen_cap = 0;
-    uint32_t *pg_blk = nullptr;      // blockpos | blkoff | ntok | lfreq
+    uint32_t *pg_blk = nullptr;      // blkoff (64-bit) | blockpos | ntok | lfreq | tile arrays
     size_t pg_blk_cap = 0;
     p2ppng::BlockInfo *pg_info = nullptr;
     size_t pg_info_cap = 0;

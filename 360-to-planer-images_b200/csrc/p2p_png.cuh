@@ -809,7 +809,9 @@ png_tree_kernel(const uint32_t *__restrict__ lfreq, const uint32_t *__restrict__
 //     f(off) = align ? roundup8(off + a) + c : off + c,
 // and that family is closed under composition (roundup8(x + y) = x + roundup8(y) for x a multiple of 8), so the offsets are
 // one prefix "sum" over function composition: every lane composes its contiguous share of the blocks, the warp scans the
-// 32 composites, every lane walks its share again from its start offset.
+// 32 composites, every lane walks its share again from its start offset.  Offsets are 64-bit throughout, blkoff[] included:
+// an image of up to 2^31 filtered bytes stored uncompressed makes a stream of more than 2^32 bits (from N > 2^29 bytes of
+// noise on), and a 32-bit block offset would put the blocks behind that point at their offset mod 2^32.
 struct OffFn {
     uint32_t align;
     unsigned long long a, c;
@@ -839,7 +841,7 @@ __device__ __forceinline__ OffFn off_of_block(const BlockInfo &bi) {
 }
 
 __global__ void __launch_bounds__(32)
-png_layout_kernel(BlockInfo *__restrict__ info, const uint32_t *__restrict__ ntok, uint32_t *__restrict__ blkoff,
+png_layout_kernel(BlockInfo *__restrict__ info, const uint32_t *__restrict__ ntok, unsigned long long *__restrict__ blkoff,
                   unsigned long long *__restrict__ zbits, const Geom G) {
     const int img = blockIdx.x, lane = threadIdx.x;
     const uint32_t nblk = ntok[img] / (uint32_t)kSymPerBlock + 1u;
@@ -864,7 +866,7 @@ png_layout_kernel(BlockInfo *__restrict__ info, const uint32_t *__restrict__ nto
     ex.c = __shfl_up_sync(0xffffffffu, inc.c, 1);
     unsigned long long off = lane ? ex(16ull) : 16ull;   // the stream starts after CMF + FLG
     for (uint32_t b = b0; b < b1; ++b) {
-        blkoff[(size_t)img * G.max_blk + b] = (uint32_t)off;
+        blkoff[(size_t)img * G.max_blk + b] = off;
         const unsigned long long next = off_of_block(bi[b])(off);
         if (bi[b].kind == 0) bi[b].bits = (uint32_t)(next - off);   // 3 + pad + 32 + 8 * len
         off = next;
@@ -895,7 +897,7 @@ constexpr int kEmitWords = kEmitTile * kMaxBits / 32 + 4;
 
 __global__ void __launch_bounds__(256)
 png_emit_kernel(const uint8_t *__restrict__ F, const uint16_t *__restrict__ tlen, const uint32_t *__restrict__ blockpos,
-                const uint32_t *__restrict__ ntok, const BlockInfo *__restrict__ info, const uint32_t *__restrict__ blkoff,
+                const uint32_t *__restrict__ ntok, const BlockInfo *__restrict__ info, const unsigned long long *__restrict__ blkoff,
                 const unsigned long long *__restrict__ zbits, uint32_t *__restrict__ Z, const Geom G) {
     // the first piece of every possible token, ready to place: bits | length << 24; [0, 256) literal bytes, [256, 512)
     // match lengths 3 .. 258 (length code + extra bits) - one shared-memory look-up per position whatever it holds

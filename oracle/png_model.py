@@ -48,12 +48,14 @@ class BitOut:
         self.acc |= (value & ((1 << length) - 1)) << self.n; self.n += length
         while self.n >= 8:
             self.buf.append(self.acc & 0xFF); self.acc >>= 8; self.n -= 8
+    def tell(self): return 8 * len(self.buf) + self.n
     def windup(self):
         if self.n: self.buf.append(self.acc & 0xFF)
         self.acc = 0; self.n = 0
 
 def build_tree(freq, elems, stree_len, extra, base, max_length, st):
-    """returns (lens, codes, max_code); st = dict with opt_len/static_len updated"""
+    """returns (lens, codes, max_code); st = dict with opt_len/static_len updated, st['overflow'] = gen_bitlen's count of
+    nodes deeper than max_length (0: the tree needed no repair)"""
     Freq = list(freq) + [0]*(HEAP_SIZE)   # room for internal nodes
     Len = [0]*(len(Freq)); Dad = [0]*len(Freq); depth = [0]*len(Freq)
     heap = [0]*(HEAP_SIZE+1); heap_len = 0; heap_max = HEAP_SIZE; max_code = -1
@@ -104,6 +106,7 @@ def build_tree(freq, elems, stree_len, extra, base, max_length, st):
             f = Freq[n]; st['opt_len'] += f * (bits + xbits)
             if stree_len is not None: st['static_len'] += f * (stree_len[n] + xbits)
         h += 1
+    st['overflow'] = overflow
     if overflow > 0:
         while True:
             bits = max_length - 1
@@ -187,7 +190,9 @@ def tokenize_rle(data):
         else: toks.append(('L', data[i])); i += 1
     return toks
 
-def flush_block(out, toks, stored_bytes, last, buf_available=True):
+def flush_block(out, toks, stored_bytes, last, buf_available=True, rec=None):
+    """_tr_flush_block; returns the block kind.  ``rec`` (a dict) receives the block's record, see ``deflate_rle``."""
+    start = out.tell()
     lfreq = [0]*L_CODES; dfreq = [0]*D_CODES
     lfreq[END_BLOCK] = 1
     for t, v in toks:
@@ -196,10 +201,15 @@ def flush_block(out, toks, stored_bytes, last, buf_available=True):
             lfreq[length_code[v-3] + LITERALS + 1] += 1; dfreq[0] += 1
     st = {'opt_len': 0, 'static_len': 0}
     llen, lcode, lmax = build_tree(lfreq, L_CODES, static_l_len, extra_lbits, LITERALS+1, MAX_BITS, st)
+    l_overflow = st['overflow']
     dlen, dcode, dmax = build_tree(dfreq, D_CODES, static_d_len, extra_dbits, 0, MAX_BITS, st)
     blfreq = [0]*BL_CODES
     scan_tree(llen, lmax, blfreq); scan_tree(dlen, dmax, blfreq)
     bllen, blcode, _ = build_tree(blfreq, BL_CODES, None, extra_blbits, 0, 7, st)
+    if rec is not None:
+        rec.update(tokens=len(toks), bytes=len(stored_bytes), start_bit=start, l_overflow=l_overflow,
+                   bl_overflow=st['overflow'], hdr_bits=0, last=last,
+                   lengths=sorted({v for t, v in toks if t == 'M'}), lmax=lmax)
     max_blindex = BL_CODES - 1
     while max_blindex >= 3 and bllen[bl_order[max_blindex]] == 0: max_blindex -= 1
     st['opt_len'] += 3*(max_blindex+1) + 5 + 5 + 4
@@ -208,6 +218,7 @@ def flush_block(out, toks, stored_bytes, last, buf_available=True):
     if len(stored_bytes) + 4 <= opt_lenb and buf_available:
         out.send((0 << 1) + last, 3); out.windup()
         L = len(stored_bytes); out.buf += bytes([L & 0xFF, L >> 8, (~L) & 0xFF, ((~L) >> 8) & 0xFF]); out.buf += stored_bytes
+        if rec is not None: rec['kind'] = 'stored'
         return 'stored'
     if static_lenb == opt_lenb:
         out.send((1 << 1) + last, 3)
@@ -228,6 +239,7 @@ def flush_block(out, toks, stored_bytes, last, buf_available=True):
         send_tree(out, llen, lmax, bllen, blcode); send_tree(out, dlen, dmax, bllen, blcode)
         ll, lc, dl, dc = llen, lcode, dlen, dcode
         kind = 'dynamic'
+        if rec is not None: rec['hdr_bits'] = out.tell() - start
     for t, v in toks:
         if t == 'L': out.send(lc[v], ll[v])
         else:
@@ -236,9 +248,16 @@ def flush_block(out, toks, stored_bytes, last, buf_available=True):
             if extra_lbits[code]: out.send(v - 3 - base_length[code], extra_lbits[code])
             out.send(dc[0], dl[0])
     out.send(lc[END_BLOCK], ll[END_BLOCK])
+    if rec is not None: rec['kind'] = kind
     return kind
 
-def deflate_rle(data, lit_bufsize=16384):
+def deflate_rle(data, lit_bufsize=16384, stats=None):
+    """(zlib stream, block kinds).  ``stats``, if a list, receives one dict per deflate block: ``kind`` ('stored', 'static'
+    or 'dynamic'), ``tokens`` and ``bytes`` (symbols and input bytes of the block, END_BLOCK not counted), ``l_overflow``
+    and ``bl_overflow`` (gen_bitlen's overflow count of the literal / length and of the bit-length tree: > 0 when the tree
+    was deeper than 15 / 7 bits and got repaired), ``hdr_bits`` (3 block-type bits + tree description of a dynamic block,
+    else 0), ``start_bit`` (bit offset of the block in the stream, the 16 bits of CMF / FLG included), ``last``, ``lmax``
+    (the largest literal / length symbol used) and ``lengths`` (the match lengths it holds)."""
     out = BitOut(); out.buf += b'\x78\x01'
     toks = tokenize_rle(data)
     sym_end = lit_bufsize - 1
@@ -249,10 +268,11 @@ def deflate_rle(data, lit_bufsize=16384):
         nbytes = sum(1 if t == 'L' else v for t, v in blk)
         full = len(blk) == sym_end
         i += len(blk)
-        if full:
-            kinds.append(flush_block(out, blk, data[pos:pos+nbytes], 0)); pos += nbytes
-            continue
-        kinds.append(flush_block(out, blk, data[pos:pos+nbytes], 1)); out.windup(); break
+        rec = {} if stats is not None else None
+        kinds.append(flush_block(out, blk, data[pos:pos+nbytes], 0 if full else 1, rec=rec)); pos += nbytes
+        if rec is not None: stats.append(rec)
+        if full: continue
+        out.windup(); break
     a = zlib.adler32(data)
     out.buf += a.to_bytes(4, 'big')
     return bytes(out.buf), kinds
