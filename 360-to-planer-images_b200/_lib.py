@@ -51,6 +51,12 @@ SIGNATURES = {
     "p2p_project_views_table": (_i, [_vp, _i, _i, C.POINTER(_i32p), C.POINTER(_i32p), _i, _pcp, _i, _i, _u8p, _i]),
     "p2p_project_batch": (_i, [_vp, _i, _i32p, _i, _i32p, _i, _pcp, _i, _i, C.POINTER(_vp), _i]),
     "p2p_project_view_list": (_i, [_vp, _i, _i, _i32p, _pcp, _i, _i, _i, _i, _u8p, _i]),
+    "p2p_project_view_list_tables": (_i, [_vp, _i, _i, _i32p, C.POINTER(_i32p), C.POINTER(_i32p), _pcp, _i, _i, _i, _i,
+                                          _u8p, _i]),
+    "p2p_process_view_list_jpeg": (_i, [_vp, _i, _u8p, _i, _i, _sz, _i, _i32p, C.POINTER(_i32p), C.POINTER(_i32p), _pcp,
+                                        _i, _i, _i, _u8p, _sz, C.POINTER(_sz)]),
+    "p2p_process_view_list_png": (_i, [_vp, _i, _u8p, _i, _i, _sz, _i, _i32p, C.POINTER(_i32p), C.POINTER(_i32p), _pcp,
+                                       _i, _i, _u8p, _sz, C.POINTER(_sz), _u8p]),
     "p2p_copy_pano": (_i, [_vp, _i, _vp, _i]),
     "p2p_upload_pano_rows": (_i, [_vp, _i, _u8p, _i, _i, _sz, _i, _i]),
     "p2p_copy_pano_rows": (_i, [_vp, _i, _vp, _i, _i, _i]),

@@ -304,26 +304,59 @@ class Projector:
         return out
 
     def project_any(self, slot: int, tables, consts, W: int, H: int, out: np.ndarray | None = None) -> np.ndarray:
-        """All yaw x pitch views of the (whole) panorama resident in ``slot`` into the host array ``out``
-        [n_yaw, n_pitch, H, W, 3]: integer-roll yaws through :meth:`project`, the others through :meth:`project_tables`,
-        from the same slot.  ``tables[k]`` = :func:`yaw_table` of yaw k.  Synchronous."""
+        """All yaw x pitch views of the panorama resident in ``slot`` into the host array ``out``
+        [n_yaw, n_pitch, H, W, 3]: integer-roll yaws only through :meth:`project`; with fractional yaws the whole yaw x pitch
+        list is one :meth:`project_list_tables` call (integer rolls and tables, at most two launches, no host wait between
+        them).  ``tables[k]`` = :func:`yaw_table` of yaw k.  Synchronous."""
         if out is None:
             out = np.empty((len(tables), len(consts), H, W, 3), np.uint8)
-        roll = [k for k, t in enumerate(tables) if t[2] is not None]
-        frac = [k for k, t in enumerate(tables) if t[2] is None]
-        tmp = ftmp = None
-        if roll:
-            tmp = self.project(slot, [tables[k][2] for k in roll], consts, W, H, out=out if not frac else None)
-        if frac:   # one pass from the same slot (round 1 materialised a rotated panorama per fractional yaw)
-            if roll:
-                self.sync(slot)   # both launches stage their host output through the slot's device buffer
-            ftmp = self.project_tables(slot, [tables[k] for k in frac], consts, W, H, out=out if not roll else None)
+        if all(t[2] is not None for t in tables):
+            self.project(slot, [t[2] for t in tables], consts, W, H, out=out)
+        else:
+            flat_tables = [t for t in tables for _ in consts]
+            self.project_list_tables(slot, flat_tables, list(consts) * len(tables), W, H, out=out.reshape(-1, H, W, 3))
         self.sync(slot)
-        if roll and frac:
-            for i, k in enumerate(roll):
-                out[k] = tmp[i]
-            for i, k in enumerate(frac):
-                out[k] = ftmp[i]
+        return out
+
+    @staticmethod
+    def _view_tables(tables):
+        """ABI form of a flat list of yaws, ``tables[i]`` = :func:`yaw_table` of view i: (yaw_shift with -1 for a
+        fractional yaw, ix / fx pointer arrays - NULL for integer rolls, one pointer per distinct table object so that views
+        of one yaw share a device table -, the arrays the pointers refer to)."""
+        P = C.POINTER(C.c_int32)
+        n = len(tables)
+        shifts = np.array([-1 if t[2] is None else t[2] for t in tables], np.int32)
+        ixp, fxp = (P * n)(), (P * n)()
+        keep = []
+        for i, t in enumerate(tables):
+            if t[2] is None:
+                ix, fx = np.ascontiguousarray(t[0], np.int32), np.ascontiguousarray(t[1], np.int32)
+                keep += [ix, fx]
+                ixp[i], fxp[i] = ix.ctypes.data_as(P), fx.ctypes.data_as(P)
+        return shifts, ixp, fxp, keep
+
+    def project_list_tables(self, slot: int, tables, consts, W: int, H: int, rows=None, out=None,
+                            out_device_ptr: int | None = None):
+        """:meth:`project_list` for any yaws: view i = (``tables[i]``, ``consts[i]``), ``tables[i]`` = :func:`yaw_table` of
+        its yaw - an integer roll or, for a fractional yaw, its column table (both remap passes of the reference per output
+        pixel, the bytes of :meth:`project_tables`).  ``rows``, ``out``, ``out_device_ptr`` as in :meth:`project_list`.
+        The slot may be partial (``process_image``, ``upload_rows``) when it holds the rows the views touch."""
+        n = len(tables)
+        if len(consts) != n:
+            raise ValueError("one pitch-constant triple per view")
+        shifts, ixp, fxp, keep = self._view_tables(tables)
+        pc = self._consts_array(consts)
+        r0, r1 = (0, H) if rows is None else (int(rows[0]), int(rows[1]))
+        if out_device_ptr is not None:
+            dst, on_dev = C.c_void_p(out_device_ptr), 1
+        else:
+            if out is None:
+                out = np.empty((n, H, W, 3), np.uint8)
+            if out.dtype != np.uint8 or not out.flags.c_contiguous or out.size != n * H * W * 3:
+                raise ValueError("out must be C-contiguous uint8 with n_views * H * W * 3 elements")
+            dst, on_dev = out.ctypes.data, 0
+        self._ck(self.lib.p2p_project_view_list_tables(self.ctx, slot, n, shifts.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                       ixp, fxp, pc, W, H, r0, r1, dst, on_dev))
         return out
 
     def project_list(self, slot: int, shifts, consts, W: int, H: int, rows=None, out=None,
@@ -555,6 +588,49 @@ class Projector:
                                                 shifts.ctypes.data_as(C.POINTER(C.c_int32)), n_pitch, pc, W, H,
                                                 buf.ctypes.data, buf.strides[0], sizes,
                                                 pixels.ctypes.data if want_pixels else None))
+        return self._files(buf, sizes, copy), pixels
+
+    # -- files of a flat list of any yaws ------------------------------------------------------------------------
+    def _pano_args(self, pano):
+        if pano is None:
+            return None, 0, 0, 0, None
+        pano = _as_u8_image(pano)
+        Hp, Wp, _ = pano.shape
+        return pano.ctypes.data, Wp, Hp, pano.strides[0], pano
+
+    def process_view_list_jpeg(self, slot: int, pano, tables, consts, W: int, H: int, quality: int = 95,
+                               copy: bool = True) -> list:
+        """JPEG files of the flat view list of :meth:`project_list_tables` (file i = view i; integer rolls and fractional
+        yaws alike): ``pano`` = None projects the panorama resident in ``slot`` (e.g. decoded there by
+        :meth:`upload_encoded`), else only the rows the views touch are uploaded.  Only the files cross PCIe.  ``copy`` as
+        in :meth:`project_jpeg`."""
+        n = len(tables)
+        shifts, ixp, fxp, keep = self._view_tables(tables)
+        pc = self._consts_array(consts)
+        src, Wp, Hp, stride, keep_pano = self._pano_args(pano)
+        buf = self._jpeg_buffer(slot, n, W, H)
+        sizes = (C.c_size_t * n)()
+        self._ck(self.lib.p2p_process_view_list_jpeg(self.ctx, slot, src, Wp, Hp, stride, n,
+                                                     shifts.ctypes.data_as(C.POINTER(C.c_int32)), ixp, fxp, pc, W, H,
+                                                     int(quality), buf.ctypes.data, buf.strides[0], sizes))
+        return self._files(buf, sizes, copy)
+
+    def process_view_list_png(self, slot: int, pano, tables, consts, W: int, H: int, want_pixels: bool = False,
+                              copy: bool = True):
+        """PNG files of the flat view list of :meth:`project_list_tables`, like :meth:`process_view_list_jpeg`.  Returns
+        (files, pixels): pixels is the [n_views, H, W, 3] array when ``want_pixels`` (for views the device encoder did not
+        handle, see :meth:`process_image_png`)."""
+        n = len(tables)
+        shifts, ixp, fxp, keep = self._view_tables(tables)
+        pc = self._consts_array(consts)
+        src, Wp, Hp, stride, keep_pano = self._pano_args(pano)
+        buf = self._file_buffer(slot, n, W * H * 4 + 4096)
+        sizes = (C.c_size_t * n)()
+        pixels = np.empty((n, H, W, 3), np.uint8) if want_pixels else None
+        self._ck(self.lib.p2p_process_view_list_png(self.ctx, slot, src, Wp, Hp, stride, n,
+                                                    shifts.ctypes.data_as(C.POINTER(C.c_int32)), ixp, fxp, pc, W, H,
+                                                    buf.ctypes.data, buf.strides[0], sizes,
+                                                    pixels.ctypes.data if want_pixels else None))
         return self._files(buf, sizes, copy), pixels
 
     # -- JPEG panoramas decoded on the device (the decode side of cv2.imread, ref :244) ----------

@@ -266,15 +266,20 @@ def _project_split(devices, src, consts, tables, yaw_angles, pitch_angles, W, H)
     n = len(projs)
     n_y, n_p = len(yaw_angles), len(pitch_angles)
     out = np.empty((n_y, n_p, H, W, 3), np.uint8)
-    flat_shifts = [tables[k][2] for k in range(n_y) for _ in range(n_p)]
+    flat_tables = [tables[k] for k in range(n_y) for _ in range(n_p)]
     flat_consts = [consts[j] for _ in range(n_y) for j in range(n_p)]
+    integer = all(t[2] is not None for t in tables)
     with contextlib.ExitStack() as stack:
         slots = _split_upload(projs, src, stack)
 
         def run(r):
             rows = shard.shard_rows(H, r, n)
-            if rows[0] < rows[1]:
-                projs[r].project_list(slots[r], flat_shifts, flat_consts, W, H, rows=rows, out=out.reshape(-1, H, W, 3))
+            if rows[0] < rows[1] and integer:
+                projs[r].project_list(slots[r], [t[2] for t in flat_tables], flat_consts, W, H, rows=rows,
+                                      out=out.reshape(-1, H, W, 3))
+            elif rows[0] < rows[1]:
+                projs[r].project_list_tables(slots[r], flat_tables, flat_consts, W, H, rows=rows,
+                                             out=out.reshape(-1, H, W, 3))
             projs[r].sync(slots[r])
 
         with ThreadPoolExecutor(max_workers=n) as ex:
@@ -292,10 +297,23 @@ def _project_files_split(devices, fmt, src, consts, tables, yaw_angles, pitch_an
     n = len(projs)
     n_y, n_p = len(yaw_angles), len(pitch_angles)
     files = [[None] * n_p for _ in range(n_y)]
+    integer = all(t[2] is not None for t in tables)
     with contextlib.ExitStack() as stack:
         slots = _split_upload(projs, src, stack)
 
         def run(r):
+            if not integer:   # fractional yaws: the device's whole run of views is one call of the view-list file entry
+                views = shard.shard_views(n_y, n_p, r, n)
+                if views:
+                    vt, vc = [tables[k] for k, _ in views], [consts[j] for _, j in views]
+                    if fmt == "png":
+                        got = projs[r].process_view_list_png(slots[r], None, vt, vc, W, H)[0]
+                    else:
+                        got = projs[r].process_view_list_jpeg(slots[r], None, vt, vc, W, H)
+                    for (k, j), f in zip(views, got):
+                        files[k][j] = f
+                projs[r].sync(slots[r])
+                return
             for j, ks in shard.group_by_pitch(shard.shard_views(n_y, n_p, r, n)).items():
                 shifts = [tables[k][2] for k in ks]
                 if fmt == "png":
@@ -312,11 +330,12 @@ def _project_files_split(devices, fmt, src, consts, tables, yaw_angles, pitch_an
 
 
 def _split_devices(devices, tables, yaw_angles, pitch_angles):
-    """The device list if this call is to be split over several GPUs (integer-roll yaws only), else None."""
+    """The device list if this call is to be split over several GPUs (any yaws: integer rolls and column tables), else
+    None."""
     devs = _default_devices if devices is None else ([int(d) for d in devices] if devices else None)
     if not devs or len(devs) < 2 or not yaw_angles or not pitch_angles:
         return None
-    return devs if all(t[2] is not None for t in tables) else None
+    return devs
 
 
 _ENCODER_FALLBACK_CODES = (-3, -5)   # P2P_ERR_NOMEM, P2P_ERR_LIMIT
@@ -365,8 +384,38 @@ def _project_jpeg(proj, pano_image, yaw_angles, pitch_angles, output_width, outp
                 flat = proj.process_image_jpeg(s, pano, shifts, consts, output_width, output_height, copy=lease is None)
         n_p = len(pitch_angles)
         return [flat[k * n_p:(k + 1) * n_p] for k in range(len(yaw_angles))]
-    return proj.project_image_jpeg(_decode_source(proj, src), yaw_angles, pitch_angles, output_width, output_height,
-                                   fov_deg, consts=consts, tables=tables)
+    if not yaw_angles or not pitch_angles:
+        return [[] for _ in yaw_angles]
+    flat, _ = _files_any_yaw(proj, "jpg", src, consts, tables, output_width, output_height, lease)
+    n_p = len(pitch_angles)
+    return [flat[k * n_p:(k + 1) * n_p] for k in range(len(yaw_angles))]
+
+
+def _files_any_yaw(proj, fmt, src, consts, tables, W, H, lease):
+    """(files, views) of all yaw x pitch views (yaw-major) when some yaws are fractional: the view-list file entries project
+    (integer rolls and column tables) and encode on the device from a slot that holds the panorama - decoded there from the
+    file, or only the rows the views touch uploaded from host pixels - so no pixels cross PCIe.  ``views`` [n_yaw, n_pitch,
+    H, W, 3] is read back only when the PNG encoder left a view to ``cv2.imwrite`` (None otherwise)."""
+    flat_t = [t for t in tables for _ in consts]
+    flat_c = list(consts) * len(tables)
+    with _slot(proj, lease) as (s,):
+        pano = src
+        if isinstance(src, _JpegSource):
+            try:
+                proj.upload_encoded(s, src.data)
+                pano = None                          # the panorama is resident in the slot
+            except _engine.P2PError as e:
+                if e.code not in _DECLINED:
+                    raise
+                pano = _decode_source(proj, src, slot=s, device_declined=True)
+        if fmt != "png":
+            return proj.process_view_list_jpeg(s, pano, flat_t, flat_c, W, H, copy=lease is None), None
+        flat, _ = proj.process_view_list_png(s, pano, flat_t, flat_c, W, H, copy=lease is None)
+        views = None
+        if any(f is None for f in flat):
+            views = proj.project_list_tables(s, flat_t, flat_c, W, H).reshape(len(tables), len(consts), H, W, 3)
+            proj.sync(s)
+        return flat, views
 
 
 def _project_png(proj, pano_image, yaw_angles, pitch_angles, output_width, output_height, fov_deg, lease=None,
@@ -404,9 +453,9 @@ def _project_png(proj, pano_image, yaw_angles, pitch_angles, output_width, outpu
                 views = proj.project(s, shifts, consts, output_width, output_height)
                 proj.sync(s)
         return [flat[k * n_p:(k + 1) * n_p] for k in range(len(yaw_angles))], views
-    views = proj.project_image(_decode_source(proj, src), yaw_angles, pitch_angles, output_width, output_height, fov_deg,
-                               consts=consts, tables=tables)
-    flat = proj.encode_png(views.reshape(-1, output_height, output_width, 3)) if views.size else []
+    if not yaw_angles or not pitch_angles:
+        return [[] for _ in yaw_angles], np.empty((len(yaw_angles), n_p, output_height, output_width, 3), np.uint8)
+    flat, views = _files_any_yaw(proj, "png", src, consts, tables, output_width, output_height, lease)
     return [flat[k * n_p:(k + 1) * n_p] for k in range(len(yaw_angles))], views
 
 

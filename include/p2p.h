@@ -182,6 +182,18 @@ int p2p_project_batch(p2p_ctx *ctx, int n_images, const int32_t *slots, int n_ya
 int p2p_project_view_list(p2p_ctx *ctx, int slot, int n_views, const int32_t *yaw_shift, const p2p_pitch_consts *pitch,
                           int W, int H, int row_begin, int row_end, uint8_t *out, int out_on_device);
 
+/* p2p_project_view_list for any yaw: view i is the integer roll yaw_shift[i] in [0, Wp), or, if yaw_shift[i] < 0, the
+ * Wp-entry column table (ix[i], fx[i]) of p2p_yaw_table (ref :79-108, :191-199, :212-218) - both remap passes of the
+ * reference per output pixel, the bytes of p2p_project_views_table.  ix / fx may be NULL when no shift is negative, and
+ * their entries of integer-roll views are not read.  Views that pass the same table pointers share one device table; views
+ * with bit-identical pitch constants share a coordinate evaluation (up to 4 per group).  The table views go out in a second
+ * launch behind the integer rolls on the slot's stream (row-segment kernel; other geometries: one launch per view).  A
+ * partial slot (p2p_process_image) serves the views whose rows it holds (the yaw pass reads the view's own rows only:
+ * p2p_view_row_range), else P2P_ERR_STATE.  Table views need the fixed-point interpolation mode (P2P_OPT_INTERP = 0). */
+int p2p_project_view_list_tables(p2p_ctx *ctx, int slot, int n_views, const int32_t *yaw_shift,
+                                 const int32_t *const *ix, const int32_t *const *fx, const p2p_pitch_consts *pitch,
+                                 int W, int H, int row_begin, int row_end, uint8_t *out, int out_on_device);
+
 /* Replicate the (possibly partial) panorama held by src's slot into dst's slot; the two contexts may live on different
  * devices of one box (cudaMemcpyPeerAsync: NVLink when peer access is available, staged by the driver otherwise) - one
  * PCIe upload plus peer copies instead of one upload per GPU when a single image is split over GPUs (SURVEY 5, 8e).
@@ -253,6 +265,20 @@ int p2p_encode_png(p2p_ctx *ctx, int slot, const uint8_t *bgr, int on_device, in
 int p2p_process_image_png(p2p_ctx *ctx, int slot, const uint8_t *bgr, int Wp, int Hp, size_t row_stride, int n_yaw,
                           const int32_t *yaw_shift, int n_pitch, const p2p_pitch_consts *pitch, int W, int H,
                           uint8_t *out_host, size_t out_stride, size_t *sizes, uint8_t *pixels_host);
+
+/* The files of a flat view list of any yaws (p2p_project_view_list_tables): view i -> file i, encoded on the device like
+ * p2p_process_image_jpeg / _png.  bgr == NULL: the panorama resident in the slot (e.g. decoded there by
+ * p2p_upload_pano_jpeg / _png, which may also be a partial slot covering the views); else only the rows the views touch
+ * are uploaded (P2P_OPT_PARTIAL_UPLOAD).  Fractional yaws then move no pixels over PCIe either.  Synchronous for this
+ * slot; pixels_host (optional, n_views * H * W * 3 bytes) as in p2p_process_image_png. */
+int p2p_process_view_list_jpeg(p2p_ctx *ctx, int slot, const uint8_t *bgr, int Wp, int Hp, size_t row_stride, int n_views,
+                               const int32_t *yaw_shift, const int32_t *const *ix, const int32_t *const *fx,
+                               const p2p_pitch_consts *pitch, int W, int H, int quality, uint8_t *out_host,
+                               size_t out_stride, size_t *sizes);
+int p2p_process_view_list_png(p2p_ctx *ctx, int slot, const uint8_t *bgr, int Wp, int Hp, size_t row_stride, int n_views,
+                              const int32_t *yaw_shift, const int32_t *const *ix, const int32_t *const *fx,
+                              const p2p_pitch_consts *pitch, int W, int H, uint8_t *out_host, size_t out_stride,
+                              size_t *sizes, uint8_t *pixels_host);
 
 /* ---- JPEG panoramas decoded on the device (replaces cv2.imread(path) of a .jpg / .jpeg input, ref :244) ---- */
 /* Headers only: size of the image if the file is in the supported subset (8-bit YCbCr 4:4:4 / 4:2:2 / 4:2:0 or
