@@ -100,6 +100,7 @@ OPT_SEG_CHUNKS = 11
 OPT_SEAM_WRAP = 12
 OPT_HOST_WAIT = 13
 OPT_PNG_FORMATS = 14
+OPT_PNG_HOST_BLOCKS = 15
 
 _lib = None
 

@@ -226,6 +226,7 @@ int p2p_get_option(p2p_ctx *ctx, int key, int *value) {
         case P2P_OPT_HOST_WAIT: *value = ctx->opt_host_wait.load(); return P2P_OK;
         case P2P_OPT_PNG_FORMATS: *value = ctx->opt_png_formats.load(); return P2P_OK;
         case P2P_OPT_GPU_HUFFMAN_COUNT: *value = (int)ctx->gpu_huffman_used; return P2P_OK;
+        case P2P_OPT_PNG_HOST_BLOCKS: *value = (int)ctx->png_host_blocks.load(); return P2P_OK;
 
         default: return fail(ctx, P2P_ERR_INVALID, "unknown option");
     }

@@ -180,6 +180,7 @@ struct p2p_ctx {
     std::atomic<int> opt_host_wait{0};   // 1: host threads sleep while they wait for a slot's stream (see wait_slot)
     std::atomic<int> opt_png_formats{0}; // PNG decoder subset (parse_png): 0 = 8-bit non-interlaced, 1 = every PNG format
     long long gpu_huffman_used = 0, gpu_huffman_fallback = 0;
+    std::atomic<long long> png_host_blocks{0};   // dynamic PNG deflate blocks the chain walk measured because the search missed them
     uint32_t *d_crc_table = nullptr;    // CRC-32 table of the PNG encoder
     p2pjpeg::Tables *d_jtab = nullptr;  // JPEG tables + header of (jW, jH, jQ): the entry of jtabs in use
     int jW = 0, jH = 0, jQ = 0;

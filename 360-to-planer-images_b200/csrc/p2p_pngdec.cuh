@@ -828,8 +828,9 @@ struct Match {            // a back-reference of a block: `len` bytes at offset 
 // Chain walk (host): from the first block behind the zlib header, through measured candidates where there are any and
 // measuring the other blocks (stored, fixed, or dynamic ones the search was not given) with the block decoder itself.
 // host_budget bounds the bits the host decodes that way, max_blocks the length of the chain.  0 = ok (blocks filled, *end_bit = end of the deflate data).
+// *host_dynamic (optional) grows by the dynamic-Huffman blocks the walk measured itself: blocks the search should have found.
 inline int walk_chain(const uint32_t *zs, const Parsed &P, std::vector<Cand> &cands, std::vector<Block> &blocks,
-                      uint64_t host_budget, uint64_t *end_bit, size_t max_blocks = (size_t)1 << 24) {
+                      uint64_t host_budget, uint64_t *end_bit, size_t max_blocks = (size_t)1 << 24, uint64_t *host_dynamic = nullptr) {
     const Info &I = P.info;
     const uint64_t n_words = stream_words(P), stream_bits = (uint64_t)(I.stream_len - 4) * 8;  // the Adler-32 is not deflate data
     std::sort(cands.begin(), cands.end(), [](const Cand &a, const Cand &b) { return a.bit < b.bit; });
@@ -851,8 +852,10 @@ inline int walk_chain(const uint32_t *zs, const Parsed &P, std::vector<Cand> &ca
             fin = it->status >> 8;
         } else {
             BlockOut R;
-            const bool stored = ((window64(zs, n_words, bit) >> 1) & 3) == 0;   // (a stored block costs nothing to measure)
+            const uint64_t btype = (window64(zs, n_words, bit) >> 1) & 3;
+            const bool stored = btype == 0;   // (a stored block costs nothing to measure)
             if (!stored && spent > host_budget) return 1;
+            if (btype == 2 && host_dynamic) ++*host_dynamic;
             if (decode_block<false>(zs, n_words, stream_bits, bit, T, lens, nullptr, nullptr, 0, I.raw_bytes, I.wsize, R)) return 1;
             if (!stored) spent += R.end_bit - bit;
             end = R.end_bit;

@@ -96,6 +96,10 @@ typedef enum p2p_option {
                                      1: also 1/2/4/16-bit gray, 16-bit RGB / gray + alpha / RGBA, palette images (1/2/4/8
                                      bit) and Adam7 interlacing, tRNS on gray / RGB / palette images - with the pixels
                                      cv2.imread's IMREAD_COLOR returns (high byte of 16-bit samples, palette alpha dropped) */
+    ,P2P_OPT_PNG_HOST_BLOCKS = 15  /* read-only: dynamic-Huffman deflate blocks of PNG inputs so far that the device's block-start
+                                     search did not return, so the host's chain walk measured them itself (stored and fixed
+                                     blocks, which the search never looks for, are not counted).  0 for files whose every
+                                     dynamic block was found */
     ,P2P_OPT_SEG_CHUNKS = 11       /* row-segment kernel: chunks of 32 pixel pairs per warp (default 4, 1..64) */
     ,P2P_OPT_PARTIAL_UPLOAD = 8    /* 1 (default): p2p_process_image copies only the panorama rows its views can
                                      touch (p2p_view_row_range) over PCIe; 0: always the whole panorama */
