@@ -206,7 +206,10 @@ struct Parsed {
     int cid[3] = {0, 0, 0};     // component ids of the frame header
 };
 
-// one DHT segment into the table sets (jdmarker.c get_dht + jdhuff.c jpeg_make_d_derived_tbl's checks); 0 = ok
+// one DHT segment into the table sets (jdmarker.c get_dht); 0 = ok.  jdhuff.c jpeg_make_d_derived_tbl checks a table when
+// a scan starts to use it, not when it is defined: a table that breaks its rules (an over-subscribed code length, a DC
+// symbol above 15) is kept as absent, and a scan that uses it is declined - a progressive file may leave such a table in
+// a slot its later scans redefine before they use it.
 inline int parse_dht(const uint8_t *seg, size_t sl, HuffTable *dc, HuffTable *ac) {
     size_t j = 0;
     while (j < sl) {
@@ -215,10 +218,11 @@ inline int parse_dht(const uint8_t *seg, size_t sl, HuffTable *dc, HuffTable *ac
         int nv = 0;
         for (int k = 0; k < 16; ++k) nv += seg[j + 1 + k];
         if (tc > 1 || th > 3 || nv > 256 || j + 17 + nv > sl) return 1;
-        if (!tc)   // jdhuff.c jpeg_make_d_derived_tbl: DC symbols are categories 0..15
-            for (int k = 0; k < nv; ++k)
-                if (seg[j + 17 + k] > 15) return 1;
-        if (!build_huff(seg + j + 1, seg + j + 17, nv, tc ? ac[th] : dc[th])) return 1;
+        HuffTable &t = tc ? ac[th] : dc[th];
+        bool ok = build_huff(seg + j + 1, seg + j + 17, nv, t);
+        if (!tc)   // DC symbols are categories 0..15
+            for (int k = 0; k < nv; ++k) ok = ok && seg[j + 17 + k] <= 15;
+        t.present = ok;
         j += 17 + (size_t)nv;
     }
     return 0;
@@ -416,6 +420,7 @@ inline int decode_progressive_scan(const uint8_t *d, const Info &I, const ProgSc
                     br.n = 0;
                     br.marker = false;
                     br.zero_bits = 0;
+                    while (br.p + 2 <= br.end && br.p[0] == 0xFF && br.p[1] == 0xFF) ++br.p;   // fill bytes
                     if (br.p + 2 > br.end || br.p[0] != 0xFF || br.p[1] != 0xD0 + next_rst) return 1;
                     next_rst = (next_rst + 1) & 7;
                     br.p += 2;
@@ -597,16 +602,20 @@ inline int decode_progressive(const uint8_t *d, size_t len, const Parsed &P, int
                 S.table[k] = t;
             }
         }
-        // the scan's data runs to the next marker that is neither a stuffed zero nor a restart marker
+        // the scan's data runs to the next marker that is neither a stuffed zero nor a restart marker; `end` is the first
+        // 0xFF in front of that marker, fill bytes included (jdmarker.c next_marker skips them), which is where the bit
+        // reader stops
         S.data = i;
         size_t e = i;
         for (;;) {
             const uint8_t *ff = static_cast<const uint8_t *>(memchr(d + e, 0xFF, len - e));
-            if (!ff || ff + 1 >= d + len) return 1;                        // no marker behind the scan: truncated
+            if (!ff) return 1;                                             // no marker behind the scan: truncated
             e = (size_t)(ff - d);
-            const uint8_t nx = ff[1];
-            if (nx == 0x00 || (nx >= 0xD0 && nx <= 0xD7)) e += 2;
-            else if (nx == 0xFF) e += 1;
+            size_t f = e;                                                  // the last 0xFF of the run
+            while (f + 1 < len && d[f + 1] == 0xFF) ++f;
+            if (f + 1 >= len) return 1;
+            const uint8_t nx = d[f + 1];
+            if (nx == 0x00 || (nx >= 0xD0 && nx <= 0xD7)) e = f + 2;
             else break;
         }
         S.end = e;

@@ -4,7 +4,8 @@
 //   nvcc -O1 -g -Xcompiler -fsanitize=address,-fsanitize=undefined,-fno-omit-frame-pointer \
 //        -gencode arch=compute_100a,code=sm_100a -o /tmp/asan_jpeg_host tools/asan_jpeg_host.cu -lasan -lubsan
 //   ASAN_OPTIONS=detect_leaks=0 /tmp/asan_jpeg_host damaged/*.jpg
-// (tests/test_jpeg_oracle.py::test_host_decoder_under_address_sanitizer builds and runs it on seeded damaged files)
+// (tests/test_jpeg_oracle.py::test_host_decoder_under_address_sanitizer builds and runs it on seeded damaged files,
+// tests/test_jpeg_progressive_scripts_oracle.py on progressive files of every scan script and damaged copies of them)
 #include <cstdio>
 #include <cstdlib>
 #include <vector>
