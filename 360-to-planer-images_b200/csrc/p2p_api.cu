@@ -2,7 +2,8 @@
 //   p2p_ctx.cuh          contexts, slots (stream + device buffers), error / allocation helpers
 //   p2p_api_project.inl  projection path: upload / pack, launches, view lists, replication across contexts
 //   p2p_api_jpeg.inl     JPEG encoder host side         p2p_api_jpegdec.inl  JPEG decoder host side
-//   p2p_api_png.inl      PNG encoder host side
+//   p2p_api_png.inl      PNG encoder host side          p2p_api_pngdec.inl   PNG decoder host side
+//   p2p_api_files.inl    files flows: the entry points that return encoded files (encode, project and encode)
 // and, below, life cycle, options, host helpers, streams / events and the stage-isolated debug exports.
 #include "p2p_ctx.cuh"
 
@@ -11,6 +12,7 @@
 #include "p2p_api_jpegdec.inl"
 #include "p2p_api_png.inl"
 #include "p2p_api_pngdec.inl"
+#include "p2p_api_files.inl"
 
 // ============================================================================================
 extern "C" {

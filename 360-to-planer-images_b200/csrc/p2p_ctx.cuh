@@ -263,6 +263,18 @@ cudaError_t wait_slot(p2p_ctx *ctx, Slot &s) {
     return e != cudaSuccess ? e : cudaEventSynchronize(s.wait_ev);
 }
 
+// the mapped host array the encoders write the sizes of n files to (s.j_sizes_h; the kernels see s.j_sizes_d)
+int ensure_file_sizes(p2p_ctx *ctx, Slot &s, int n) {
+    if (s.j_sizes_n >= n) return P2P_OK;
+    if (s.j_sizes_h) CK(cudaFreeHost(s.j_sizes_h));
+    s.j_sizes_h = nullptr;
+    CK(cudaHostAlloc(reinterpret_cast<void **>(&s.j_sizes_h), (size_t)n * sizeof(unsigned long long),
+                     cudaHostAllocMapped | cudaHostAllocPortable));
+    CK(cudaHostGetDevicePointer(reinterpret_cast<void **>(&s.j_sizes_d), s.j_sizes_h, 0));
+    s.j_sizes_n = n;
+    return P2P_OK;
+}
+
 int slot_ok(p2p_ctx *ctx, int slot) { return ctx && slot >= 0 && slot < ctx->n_slots; }
 
 int check_dims(p2p_ctx *ctx, int Wp, int Hp) {

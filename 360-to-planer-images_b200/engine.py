@@ -263,20 +263,25 @@ class Projector:
             arr[i].f, arr[i].c, arr[i].s = f, c, s
         return arr
 
+    @staticmethod
+    def _out_arg(out, out_device_ptr, shape):
+        """(out, destination, out_on_device) of a projection: ``out_device_ptr``, else the host array ``out`` (created with
+        ``shape`` if None), which must be C-contiguous uint8 with as many elements as ``shape``."""
+        if out_device_ptr is not None:
+            return out, C.c_void_p(out_device_ptr), 1
+        if out is None:
+            out = np.empty(shape, np.uint8)
+        if out.dtype != np.uint8 or not out.flags.c_contiguous or out.size != int(np.prod(shape)):
+            raise ValueError(f"out must be C-contiguous uint8 with {' * '.join(map(str, shape))} elements")
+        return out, out.ctypes.data, 0
+
     def project(self, slot: int, shifts, consts, W: int, H: int, out=None, out_device_ptr: int | None = None):
         """Enqueue n_yaw x n_pitch views.  ``out``: host array [n_yaw, n_pitch, H, W, 3] (created if
         None) or ``out_device_ptr`` for device-resident results.  Returns ``out`` (valid after sync)."""
         shifts = np.ascontiguousarray(shifts, np.int32)
         n_yaw, n_pitch = int(shifts.shape[0]), len(consts)
         pc = self._consts_array(consts)
-        if out_device_ptr is not None:
-            dst, on_dev = C.c_void_p(out_device_ptr), 1
-        else:
-            if out is None:
-                out = np.empty((n_yaw, n_pitch, H, W, 3), np.uint8)
-            if out.dtype != np.uint8 or not out.flags.c_contiguous or out.size != n_yaw * n_pitch * H * W * 3:
-                raise ValueError("out must be C-contiguous uint8 [n_yaw, n_pitch, H, W, 3]")
-            dst, on_dev = out.ctypes.data, 0
+        out, dst, on_dev = self._out_arg(out, out_device_ptr, (n_yaw, n_pitch, H, W, 3))
         self._ck(self.lib.p2p_project_views(self.ctx, slot, n_yaw, shifts.ctypes.data_as(C.POINTER(C.c_int32)),
                                             n_pitch, pc, W, H, dst, on_dev))
         return out
@@ -292,14 +297,7 @@ class Projector:
         P = C.POINTER(C.c_int32)
         ixp = (P * n_yaw)(*[a.ctypes.data_as(P) for a in ixs])
         fxp = (P * n_yaw)(*[a.ctypes.data_as(P) for a in fxs])
-        if out_device_ptr is not None:
-            dst, on_dev = C.c_void_p(out_device_ptr), 1
-        else:
-            if out is None:
-                out = np.empty((n_yaw, n_pitch, H, W, 3), np.uint8)
-            if out.dtype != np.uint8 or not out.flags.c_contiguous or out.size != n_yaw * n_pitch * H * W * 3:
-                raise ValueError("out must be C-contiguous uint8 [n_yaw, n_pitch, H, W, 3]")
-            dst, on_dev = out.ctypes.data, 0
+        out, dst, on_dev = self._out_arg(out, out_device_ptr, (n_yaw, n_pitch, H, W, 3))
         self._ck(self.lib.p2p_project_views_table(self.ctx, slot, n_yaw, ixp, fxp, n_pitch, pc, W, H, dst, on_dev))
         return out
 
@@ -347,14 +345,7 @@ class Projector:
         shifts, ixp, fxp, keep = self._view_tables(tables)
         pc = self._consts_array(consts)
         r0, r1 = (0, H) if rows is None else (int(rows[0]), int(rows[1]))
-        if out_device_ptr is not None:
-            dst, on_dev = C.c_void_p(out_device_ptr), 1
-        else:
-            if out is None:
-                out = np.empty((n, H, W, 3), np.uint8)
-            if out.dtype != np.uint8 or not out.flags.c_contiguous or out.size != n * H * W * 3:
-                raise ValueError("out must be C-contiguous uint8 with n_views * H * W * 3 elements")
-            dst, on_dev = out.ctypes.data, 0
+        out, dst, on_dev = self._out_arg(out, out_device_ptr, (n, H, W, 3))
         self._ck(self.lib.p2p_project_view_list_tables(self.ctx, slot, n, shifts.ctypes.data_as(C.POINTER(C.c_int32)),
                                                        ixp, fxp, pc, W, H, r0, r1, dst, on_dev))
         return out
@@ -370,14 +361,7 @@ class Projector:
             raise ValueError("one pitch-constant triple per view")
         pc = self._consts_array(consts)
         r0, r1 = (0, H) if rows is None else (int(rows[0]), int(rows[1]))
-        if out_device_ptr is not None:
-            dst, on_dev = C.c_void_p(out_device_ptr), 1
-        else:
-            if out is None:
-                out = np.empty((n, H, W, 3), np.uint8)
-            if out.dtype != np.uint8 or not out.flags.c_contiguous or out.size != n * H * W * 3:
-                raise ValueError("out must be C-contiguous uint8 with n_views * H * W * 3 elements")
-            dst, on_dev = out.ctypes.data, 0
+        out, dst, on_dev = self._out_arg(out, out_device_ptr, (n, H, W, 3))
         self._ck(self.lib.p2p_project_view_list(self.ctx, slot, n, shifts.ctypes.data_as(C.POINTER(C.c_int32)), pc, W, H,
                                                 r0, r1, dst, on_dev))
         return out
@@ -443,7 +427,7 @@ class Projector:
                                             len(consts), pc, W, H, out.ctypes.data))
         return out
 
-    # -- JPEG files (the encode side of cv2.imwrite, ref :277) ---------------------------------
+    # -- files (the encode side of cv2.imwrite, ref :277) ---------------------------------------
     def _file_buffer(self, slot: int, n: int, stride: int) -> np.ndarray:
         """page-locked [n, stride] file buffer of a slot (a slot is driven by one thread at a time)"""
         cache = self.__dict__.setdefault("_jpeg_bufs", {})
@@ -462,8 +446,24 @@ class Projector:
             return [buf[i, :sizes[i]].tobytes() if sizes[i] else None for i in range(len(sizes))]
         return [memoryview(buf[i, :sizes[i]]) if sizes[i] else None for i in range(len(sizes))]
 
-    def _jpeg_buffer(self, slot: int, n: int, W: int, H: int) -> np.ndarray:
-        return self._file_buffer(slot, n, W * H * 3 + 4096)
+    def _files_call(self, fn, slot: int, args, n: int, stride: int, copy: bool = True, pixels=()) -> list:
+        """One files entry of the ABI, ``fn(ctx, slot, *args, file_buffer, file_stride, sizes, *pixels)``: the n files land
+        in the slot's page-locked file buffer, ``stride`` bytes apart, and come back as :meth:`_files` returns them.
+        ``pixels``: the pixel output of the PNG entries that take one, ``(array or None,)``."""
+        buf = self._file_buffer(slot, n, stride)
+        sizes = (C.c_size_t * n)()
+        self._ck(fn(self.ctx, slot, *args, buf.ctypes.data, buf.strides[0], sizes,
+                    *[None if p is None else p.ctypes.data for p in pixels]))
+        return self._files(buf, sizes, copy)
+
+    @staticmethod
+    def _pano_args(pano):
+        """(pointer, Wp, Hp, row stride, array) of the optional host panorama of a files entry (None: the resident one)."""
+        if pano is None:
+            return None, 0, 0, 0, None
+        pano = _as_u8_image(pano)
+        Hp, Wp, _ = pano.shape
+        return pano.ctypes.data, Wp, Hp, pano.strides[0], pano
 
     def encode_jpeg(self, images: np.ndarray, quality: int = 95, slot: int | None = None) -> list:
         """JPEG files (bytes) of ``images`` u8 [n, H, W, 3] (BGR), encoded on the GPU; byte-identical to
@@ -474,13 +474,10 @@ class Projector:
         n, H, W, ch = images.shape
         if ch != 3:
             raise ValueError("images must be [n, H, W, 3]")
-        sizes = (C.c_size_t * n)()
 
         def run(s):
-            buf = self._jpeg_buffer(s, n, W, H)
-            self._ck(self.lib.p2p_encode_jpeg(self.ctx, s, images.ctypes.data, 0, n, W, H, int(quality),
-                                              buf.ctypes.data, buf.strides[0], sizes))
-            return [buf[i, :sizes[i]].tobytes() for i in range(n)]
+            return self._files_call(self.lib.p2p_encode_jpeg, s, (images.ctypes.data, 0, n, W, H, int(quality)), n,
+                                    W * H * 3 + 4096)
 
         if slot is None:
             with self.slots(1) as (s,):
@@ -493,31 +490,20 @@ class Projector:
         file buffer instead of bytes (valid until the slot is used again)."""
         shifts = np.ascontiguousarray(shifts, np.int32)
         n_yaw, n_pitch = int(shifts.shape[0]), len(consts)
-        n = n_yaw * n_pitch
-        pc = self._consts_array(consts)
-        buf = self._jpeg_buffer(slot, n, W, H)
-        sizes = (C.c_size_t * n)()
-        self._ck(self.lib.p2p_project_views_jpeg(self.ctx, slot, n_yaw, shifts.ctypes.data_as(C.POINTER(C.c_int32)),
-                                                 n_pitch, pc, W, H, int(quality), buf.ctypes.data, buf.strides[0], sizes))
-        return self._files(buf, sizes, copy)
+        args = (n_yaw, shifts.ctypes.data_as(C.POINTER(C.c_int32)), n_pitch, self._consts_array(consts), W, H, int(quality))
+        return self._files_call(self.lib.p2p_project_views_jpeg, slot, args, n_yaw * n_pitch, W * H * 3 + 4096, copy)
 
     def process_image_jpeg(self, slot: int, pano: np.ndarray, shifts, consts, W: int, H: int, quality: int = 95,
                            copy: bool = True) -> list:
         """upload (the rows the views touch) + project + JPEG-encode in one ABI call: the files (bytes, yaw-major;
         ``copy=False``: memoryviews of the slot's file buffer) of all n_yaw x n_pitch views.  Blocks this thread only;
         other slots keep running."""
-        pano = _as_u8_image(pano)
-        Hp, Wp, _ = pano.shape
+        src, Wp, Hp, stride, pano = self._pano_args(_as_u8_image(pano))
         shifts = np.ascontiguousarray(shifts, np.int32)
         n_yaw, n_pitch = int(shifts.shape[0]), len(consts)
-        n = n_yaw * n_pitch
-        pc = self._consts_array(consts)
-        buf = self._jpeg_buffer(slot, n, W, H)
-        sizes = (C.c_size_t * n)()
-        self._ck(self.lib.p2p_process_image_jpeg(self.ctx, slot, pano.ctypes.data, Wp, Hp, pano.strides[0], n_yaw,
-                                                 shifts.ctypes.data_as(C.POINTER(C.c_int32)), n_pitch, pc, W, H,
-                                                 int(quality), buf.ctypes.data, buf.strides[0], sizes))
-        return self._files(buf, sizes, copy)
+        args = (src, Wp, Hp, stride, n_yaw, shifts.ctypes.data_as(C.POINTER(C.c_int32)), n_pitch, self._consts_array(consts),
+                W, H, int(quality))
+        return self._files_call(self.lib.p2p_process_image_jpeg, slot, args, n_yaw * n_pitch, W * H * 3 + 4096, copy)
 
     def project_image_jpeg(self, pano: np.ndarray, yaw_angles, pitch_angles, W: int, H: int, fov_deg=90,
                            consts=None, tables=None, quality: int = 95) -> list:
@@ -552,12 +538,9 @@ class Projector:
         n, H, W, ch = images.shape
         if ch != 3:
             raise ValueError("images must be [n, H, W, 3]")
-        sizes = (C.c_size_t * n)()
 
         def run(s):
-            buf = self._file_buffer(s, n, W * H * 4 + 4096)
-            self._ck(self.lib.p2p_encode_png(self.ctx, s, images.ctypes.data, 0, n, W, H, buf.ctypes.data, buf.strides[0], sizes))
-            return [buf[i, :sizes[i]].tobytes() if sizes[i] else None for i in range(n)]
+            return self._files_call(self.lib.p2p_encode_png, s, (images.ctypes.data, 0, n, W, H), n, W * H * 4 + 4096)
 
         if slot is None:
             with self.slots(1) as (s,):
@@ -570,34 +553,17 @@ class Projector:
         Returns (files, pixels): files[i] is bytes (``copy=False``: a memoryview of the slot's page-locked file buffer,
         valid until the slot is used again) or None (view not handled by the device encoder); pixels is the
         [n_yaw, n_pitch, H, W, 3] array when ``want_pixels`` (so the caller can ``cv2.imwrite`` the None views)."""
+        src, Wp, Hp, stride, pano = self._pano_args(pano)
         shifts = np.ascontiguousarray(shifts, np.int32)
         n_yaw, n_pitch = int(shifts.shape[0]), len(consts)
-        n = n_yaw * n_pitch
-        pc = self._consts_array(consts)
-        buf = self._file_buffer(slot, n, W * H * 4 + 4096)
-        sizes = (C.c_size_t * n)()
         pixels = np.empty((n_yaw, n_pitch, H, W, 3), np.uint8) if want_pixels else None
-        if pano is not None:
-            pano = _as_u8_image(pano)
-            Hp, Wp, _ = pano.shape
-            src, stride = pano.ctypes.data, pano.strides[0]
-        else:
-            Hp = Wp = 0
-            src, stride = None, 0
-        self._ck(self.lib.p2p_process_image_png(self.ctx, slot, src, Wp, Hp, stride, n_yaw,
-                                                shifts.ctypes.data_as(C.POINTER(C.c_int32)), n_pitch, pc, W, H,
-                                                buf.ctypes.data, buf.strides[0], sizes,
-                                                pixels.ctypes.data if want_pixels else None))
-        return self._files(buf, sizes, copy), pixels
+        args = (src, Wp, Hp, stride, n_yaw, shifts.ctypes.data_as(C.POINTER(C.c_int32)), n_pitch, self._consts_array(consts),
+                W, H)
+        files = self._files_call(self.lib.p2p_process_image_png, slot, args, n_yaw * n_pitch, W * H * 4 + 4096, copy,
+                                 (pixels,))
+        return files, pixels
 
     # -- files of a flat list of any yaws ------------------------------------------------------------------------
-    def _pano_args(self, pano):
-        if pano is None:
-            return None, 0, 0, 0, None
-        pano = _as_u8_image(pano)
-        Hp, Wp, _ = pano.shape
-        return pano.ctypes.data, Wp, Hp, pano.strides[0], pano
-
     def process_view_list_jpeg(self, slot: int, pano, tables, consts, W: int, H: int, quality: int = 95,
                                copy: bool = True) -> list:
         """JPEG files of the flat view list of :meth:`project_list_tables` (file i = view i; integer rolls and fractional
@@ -606,14 +572,10 @@ class Projector:
         in :meth:`project_jpeg`."""
         n = len(tables)
         shifts, ixp, fxp, keep = self._view_tables(tables)
-        pc = self._consts_array(consts)
-        src, Wp, Hp, stride, keep_pano = self._pano_args(pano)
-        buf = self._jpeg_buffer(slot, n, W, H)
-        sizes = (C.c_size_t * n)()
-        self._ck(self.lib.p2p_process_view_list_jpeg(self.ctx, slot, src, Wp, Hp, stride, n,
-                                                     shifts.ctypes.data_as(C.POINTER(C.c_int32)), ixp, fxp, pc, W, H,
-                                                     int(quality), buf.ctypes.data, buf.strides[0], sizes))
-        return self._files(buf, sizes, copy)
+        src, Wp, Hp, stride, pano = self._pano_args(pano)
+        args = (src, Wp, Hp, stride, n, shifts.ctypes.data_as(C.POINTER(C.c_int32)), ixp, fxp, self._consts_array(consts),
+                W, H, int(quality))
+        return self._files_call(self.lib.p2p_process_view_list_jpeg, slot, args, n, W * H * 3 + 4096, copy)
 
     def process_view_list_png(self, slot: int, pano, tables, consts, W: int, H: int, want_pixels: bool = False,
                               copy: bool = True):
@@ -622,16 +584,11 @@ class Projector:
         handle, see :meth:`process_image_png`)."""
         n = len(tables)
         shifts, ixp, fxp, keep = self._view_tables(tables)
-        pc = self._consts_array(consts)
-        src, Wp, Hp, stride, keep_pano = self._pano_args(pano)
-        buf = self._file_buffer(slot, n, W * H * 4 + 4096)
-        sizes = (C.c_size_t * n)()
+        src, Wp, Hp, stride, pano = self._pano_args(pano)
         pixels = np.empty((n, H, W, 3), np.uint8) if want_pixels else None
-        self._ck(self.lib.p2p_process_view_list_png(self.ctx, slot, src, Wp, Hp, stride, n,
-                                                    shifts.ctypes.data_as(C.POINTER(C.c_int32)), ixp, fxp, pc, W, H,
-                                                    buf.ctypes.data, buf.strides[0], sizes,
-                                                    pixels.ctypes.data if want_pixels else None))
-        return self._files(buf, sizes, copy), pixels
+        args = (src, Wp, Hp, stride, n, shifts.ctypes.data_as(C.POINTER(C.c_int32)), ixp, fxp, self._consts_array(consts),
+                W, H)
+        return self._files_call(self.lib.p2p_process_view_list_png, slot, args, n, W * H * 4 + 4096, copy, (pixels,)), pixels
 
     # -- JPEG panoramas decoded on the device (the decode side of cv2.imread, ref :244) ----------
     def jpeg_probe(self, data: bytes):

@@ -171,6 +171,20 @@ def _decode_source(proj, src, slot=None, device_declined=False):
     return img
 
 
+def _resident_or_pixels(proj, slot, src):
+    """None when the panorama of ``src`` is now resident in ``slot`` (decoded there from its file), else its host pixels:
+    a host array as it is, or a file the device decoder declined (or could not fit, ``_DECLINED``) read by cv2.imread."""
+    if not isinstance(src, _JpegSource):
+        return src
+    try:
+        proj.upload_encoded(slot, src.data)
+        return None
+    except _engine.P2PError as e:
+        if e.code not in _DECLINED:
+            raise
+        return _decode_source(proj, src, slot=slot, device_declined=True)
+
+
 def _geometry(src, yaw_angles, pitch_angles, output_width, output_height, fov_deg):
     if isinstance(src, _JpegSource):
         Wp, Hp = src.Wp, src.Hp
@@ -190,14 +204,11 @@ def _project(proj, pano_image, yaw_angles, pitch_angles, output_width, output_he
     if devs:
         return _project_split(devs, src, consts, tables, yaw_angles, pitch_angles, output_width, output_height)
     if isinstance(src, _JpegSource) and yaw_angles and pitch_angles:
-        try:  # decode on the device straight into a slot, project from there (fractional yaws too: one pass, same slot)
-            with proj.slots(1) as (s,):
-                proj.upload_encoded(s, src.data)
+        # decode on the device straight into a slot, project from there (fractional yaws too: one pass, same slot)
+        with proj.slots(1) as (s,):
+            src = _resident_or_pixels(proj, s, src)
+            if src is None:
                 return proj.project_any(s, tables, consts, output_width, output_height)
-        except _engine.P2PError as e:
-            if e.code not in _DECLINED:
-                raise
-            src = _decode_source(proj, src, device_declined=True)
     return proj.project_image(_decode_source(proj, src), yaw_angles, pitch_angles, output_width, output_height, fov_deg,
                               consts=consts, tables=tables)
 
@@ -207,15 +218,7 @@ def _split_upload(projs, src, stack):
     the others with peer copies (NVLink) ordered after it on the device.  Returns the slots."""
     slots = [stack.enter_context(pr.slots(1))[0] for pr in projs]
     p0, s0 = projs[0], slots[0]
-    pano = src
-    if isinstance(src, _JpegSource):
-        try:
-            p0.upload_encoded(s0, src.data)
-            pano = None
-        except _engine.P2PError as e:
-            if e.code not in _DECLINED:
-                raise
-            pano = _decode_source(p0, src, slot=s0, device_declined=True)
+    pano = _resident_or_pixels(p0, s0, src)
     if pano is not None:
         # host pixels: every device uploads 1 / n of the rows over its own PCIe link and fetches the rest from its peers
         stack.callback(lambda keep=scatter_upload(projs, slots, pano): None)  # the host array outlives the async copies
@@ -268,16 +271,12 @@ def _project_split(devices, src, consts, tables, yaw_angles, pitch_angles, W, H)
     out = np.empty((n_y, n_p, H, W, 3), np.uint8)
     flat_tables = [tables[k] for k in range(n_y) for _ in range(n_p)]
     flat_consts = [consts[j] for _ in range(n_y) for j in range(n_p)]
-    integer = all(t[2] is not None for t in tables)
     with contextlib.ExitStack() as stack:
         slots = _split_upload(projs, src, stack)
 
         def run(r):
             rows = shard.shard_rows(H, r, n)
-            if rows[0] < rows[1] and integer:
-                projs[r].project_list(slots[r], [t[2] for t in flat_tables], flat_consts, W, H, rows=rows,
-                                      out=out.reshape(-1, H, W, 3))
-            elif rows[0] < rows[1]:
+            if rows[0] < rows[1]:   # (integer rolls and column tables alike)
                 projs[r].project_list_tables(slots[r], flat_tables, flat_consts, W, H, rows=rows,
                                              out=out.reshape(-1, H, W, 3))
             projs[r].sync(slots[r])
@@ -357,122 +356,58 @@ def _slot(proj, lease):
     return contextlib.nullcontext((s,))
 
 
-def _project_jpeg(proj, pano_image, yaw_angles, pitch_angles, output_width, output_height, fov_deg, lease=None,
-                  devices=None):
-    """[n_yaw][n_pitch] JPEG files (bytes; with a ``lease`` zero-copy views of the slot's file buffer, see ``_slot``) through
-    the device projection + encoder, using the module caches."""
+def _project_files(fmt, proj, pano_image, yaw_angles, pitch_angles, output_width, output_height, fov_deg, lease=None,
+                   devices=None):
+    """([n_yaw][n_pitch] files, views): the views projected and encoded on the device, ``fmt`` "jpg" or "png", using the
+    module caches.  Files are bytes, or with a ``lease`` zero-copy views of the slot's file buffer (see ``_slot``).  Integer
+    yaw rolls go to the product entries; with a fractional yaw the view-list entries project the integer rolls and the
+    column tables together.  The panorama is decoded into the slot from its file, or only the rows the views touch are
+    uploaded from host pixels, so no pixels cross PCIe.  A None file is a view the PNG encoder did not handle (the ABI's
+    ``sizes[i] = 0``; not produced any more): ``views`` [n_yaw, n_pitch, H, W, 3] then holds the pixels of all views so that
+    ``cv2.imwrite`` can write those, exactly as the reference would; otherwise ``views`` is None."""
+    W, H = output_width, output_height
     src = pano_image if isinstance(pano_image, _JpegSource) else _engine._as_u8_image(pano_image, "pano_image")
-    consts, tables = _geometry(src, yaw_angles, pitch_angles, output_width, output_height, fov_deg)
-    devs = _split_devices(devices, tables, yaw_angles, pitch_angles)
-    if devs:
-        return _project_files_split(devs, "jpg", src, consts, tables, yaw_angles, pitch_angles, output_width, output_height)
-    if yaw_angles and pitch_angles and all(t[2] is not None for t in tables):
-        shifts = [t[2] for t in tables]
-        with _slot(proj, lease) as (s,):
-            pano = src
-            if isinstance(src, _JpegSource):
-                try:  # JPEG in, JPEG out: no pixel ever crosses PCIe
-                    proj.upload_encoded(s, src.data)
-                    pano = None                      # the panorama is resident in the slot
-                except _engine.P2PError as e:
-                    if e.code not in _DECLINED:
-                        raise
-                    pano = _decode_source(proj, src, slot=s, device_declined=True)
-            if pano is None:
-                flat = proj.project_jpeg(s, shifts, consts, output_width, output_height, copy=lease is None)
-            else:
-                flat = proj.process_image_jpeg(s, pano, shifts, consts, output_width, output_height, copy=lease is None)
-        n_p = len(pitch_angles)
-        return [flat[k * n_p:(k + 1) * n_p] for k in range(len(yaw_angles))]
-    if not yaw_angles or not pitch_angles:
-        return [[] for _ in yaw_angles]
-    flat, _ = _files_any_yaw(proj, "jpg", src, consts, tables, output_width, output_height, lease)
-    n_p = len(pitch_angles)
-    return [flat[k * n_p:(k + 1) * n_p] for k in range(len(yaw_angles))]
-
-
-def _files_any_yaw(proj, fmt, src, consts, tables, W, H, lease):
-    """(files, views) of all yaw x pitch views (yaw-major) when some yaws are fractional: the view-list file entries project
-    (integer rolls and column tables) and encode on the device from a slot that holds the panorama - decoded there from the
-    file, or only the rows the views touch uploaded from host pixels - so no pixels cross PCIe.  ``views`` [n_yaw, n_pitch,
-    H, W, 3] is read back only when the PNG encoder left a view to ``cv2.imwrite`` (None otherwise)."""
-    flat_t = [t for t in tables for _ in consts]
-    flat_c = list(consts) * len(tables)
-    with _slot(proj, lease) as (s,):
-        pano = src
-        if isinstance(src, _JpegSource):
-            try:
-                proj.upload_encoded(s, src.data)
-                pano = None                          # the panorama is resident in the slot
-            except _engine.P2PError as e:
-                if e.code not in _DECLINED:
-                    raise
-                pano = _decode_source(proj, src, slot=s, device_declined=True)
-        if fmt != "png":
-            return proj.process_view_list_jpeg(s, pano, flat_t, flat_c, W, H, copy=lease is None), None
-        flat, _ = proj.process_view_list_png(s, pano, flat_t, flat_c, W, H, copy=lease is None)
-        views = None
-        if any(f is None for f in flat):
-            views = proj.project_list_tables(s, flat_t, flat_c, W, H).reshape(len(tables), len(consts), H, W, 3)
-            proj.sync(s)
-        return flat, views
-
-
-def _project_png(proj, pano_image, yaw_angles, pitch_angles, output_width, output_height, fov_deg, lease=None,
-                 devices=None):
-    """([n_yaw][n_pitch] PNG files (bytes; with a ``lease`` zero-copy views of the slot's file buffer, see ``_slot``) or
-    None, views or None): projection and PNG encoder on the device.  A None file
-    is a view the device encoder did not handle (the ABI's ``sizes[i] = 0``; not produced any more): ``views`` then holds the pixels
-    of all views so that ``cv2.imwrite`` can write those, exactly as the reference would."""
-    src = pano_image if isinstance(pano_image, _JpegSource) else _engine._as_u8_image(pano_image, "pano_image")
-    consts, tables = _geometry(src, yaw_angles, pitch_angles, output_width, output_height, fov_deg)
+    consts, tables = _geometry(src, yaw_angles, pitch_angles, W, H, fov_deg)
     n_p = len(pitch_angles)
     devs = _split_devices(devices, tables, yaw_angles, pitch_angles)
     if devs:
-        files = _project_files_split(devs, "png", src, consts, tables, yaw_angles, pitch_angles, output_width, output_height)
+        files = _project_files_split(devs, fmt, src, consts, tables, yaw_angles, pitch_angles, W, H)
         views = None
         if any(f is None for per_yaw in files for f in per_yaw):  # (the device encoder handles every image today)
-            views = _project_split(devs, src, consts, tables, yaw_angles, pitch_angles, output_width, output_height)
+            views = _project_split(devs, src, consts, tables, yaw_angles, pitch_angles, W, H)
         return files, views
-    if yaw_angles and pitch_angles and all(t[2] is not None for t in tables):
-        shifts = [t[2] for t in tables]
-        with _slot(proj, lease) as (s,):
-            pano = src
-            if isinstance(src, _JpegSource):
-                try:
-                    proj.upload_encoded(s, src.data)
-                    pano = None                      # the panorama is resident in the slot
-                except _engine.P2PError as e:
-                    if e.code not in _DECLINED:
-                        raise
-                    pano = _decode_source(proj, src, slot=s, device_declined=True)
-            flat, _ = proj.process_image_png(s, pano, shifts, consts, output_width, output_height, want_pixels=False,
-                                             copy=lease is None)
-            views = None
-            if any(f is None for f in flat):         # read the pixels back only when cv2 has to write some views
-                views = proj.project(s, shifts, consts, output_width, output_height)
-                proj.sync(s)
-        return [flat[k * n_p:(k + 1) * n_p] for k in range(len(yaw_angles))], views
     if not yaw_angles or not pitch_angles:
-        return [[] for _ in yaw_angles], np.empty((len(yaw_angles), n_p, output_height, output_width, 3), np.uint8)
-    flat, views = _files_any_yaw(proj, "png", src, consts, tables, output_width, output_height, lease)
+        return [[] for _ in yaw_angles], None
+    integer = all(t[2] is not None for t in tables)
+    shifts = [t[2] for t in tables]
+    flat_t = [t for t in tables for _ in consts]
+    flat_c = list(consts) * len(tables)
+    copy = lease is None
+    with _slot(proj, lease) as (s,):
+        pano = _resident_or_pixels(proj, s, src)
+        if fmt == "png" and integer:
+            flat = proj.process_image_png(s, pano, shifts, consts, W, H, want_pixels=False, copy=copy)[0]
+        elif fmt == "png":
+            flat = proj.process_view_list_png(s, pano, flat_t, flat_c, W, H, copy=copy)[0]
+        elif integer and pano is None:   # JPEG in, JPEG out: no pixel ever crosses PCIe
+            flat = proj.project_jpeg(s, shifts, consts, W, H, copy=copy)
+        elif integer:
+            flat = proj.process_image_jpeg(s, pano, shifts, consts, W, H, copy=copy)
+        else:
+            flat = proj.process_view_list_jpeg(s, pano, flat_t, flat_c, W, H, copy=copy)
+        views = None
+        if any(f is None for f in flat):         # read the pixels back only when cv2 has to write some views
+            if integer:
+                views = proj.project(s, shifts, consts, W, H)
+            else:
+                views = proj.project_list_tables(s, flat_t, flat_c, W, H).reshape(len(tables), n_p, H, W, 3)
+            proj.sync(s)
     return [flat[k * n_p:(k + 1) * n_p] for k in range(len(yaw_angles))], views
 
 
-def _save_png(cv2, files, views, base_name, output_dir, yaw_angles, pitch_angles, output_width, output_height,
-              output_format, executor):
-    """Write device-encoded PNG files; views the device encoder declined are encoded by ``cv2.imwrite`` (ref :277)."""
-
-    def save(k, i):
-        out_filename = (f"{base_name}_{output_width}x{output_height}_yaw_{yaw_angles[k]}"
-                        f"_pitch_{pitch_angles[i]}.{output_format}")
-        if files[k][i] is not None:
-            (output_dir / out_filename).write_bytes(files[k][i])
-        else:
-            cv2.imwrite(str(output_dir / out_filename), views[k, i])
-        logging.debug(f"Saved {output_dir / out_filename}")
-
-    return [_YawGroup([executor.submit(save, k, i) for i in range(len(pitch_angles))]) for k in range(len(yaw_angles))]
+def _out_path(output_dir, base_name, output_width, output_height, yaw_angle, pitch_angle, output_format):
+    """The reference's name of an output file (ref :275)."""
+    return output_dir / f"{base_name}_{output_width}x{output_height}_yaw_{yaw_angle}_pitch_{pitch_angle}.{output_format}"
 
 
 def _save_files(files, base_name, output_dir, yaw_angles, pitch_angles, output_width, output_height, output_format,
@@ -481,10 +416,10 @@ def _save_files(files, base_name, output_dir, yaw_angles, pitch_angles, output_w
 
     def save_yaw(k):
         for i in range(len(pitch_angles)):
-            out_filename = (f"{base_name}_{output_width}x{output_height}_yaw_{yaw_angles[k]}"
-                            f"_pitch_{pitch_angles[i]}.{output_format}")
-            (output_dir / out_filename).write_bytes(files[k][i])
-            logging.debug(f"Saved {output_dir / out_filename}")
+            path = _out_path(output_dir, base_name, output_width, output_height, yaw_angles[k], pitch_angles[i],
+                             output_format)
+            path.write_bytes(files[k][i])
+            logging.debug(f"Saved {path}")
 
     return [executor.submit(save_yaw, k) for k in range(len(yaw_angles))]
 
@@ -537,16 +472,15 @@ def process_single_image(input_image_path, output_dir, yaw_angles, pitch_angles,
     pitch_angles = list(pitch_angles)
     jpeg = _is_jpeg(output_format)
     png = str(output_format).lower() == "png"
+    files = None
     # the slot stays leased until the files are on disk: they are written straight from its page-locked buffer
     with contextlib.ExitStack() as lease, ThreadPoolExecutor(max_workers=max(1, int(num_workers))) as executor:
         try:
             try:
-                if jpeg:  # projected and encoded on the device: only the files come back
-                    files = _project_jpeg(get_projector(), input_image, yaw_angles, pitch_angles, output_width,
-                                          output_height, fov_deg, lease=lease, devices=devices)
-                elif png:
-                    files, views = _project_png(get_projector(), input_image, yaw_angles, pitch_angles, output_width,
-                                                output_height, fov_deg, lease=lease, devices=devices)
+                if jpeg or png:  # projected and encoded on the device: only the files come back
+                    files, views = _project_files("jpg" if jpeg else "png", get_projector(), input_image, yaw_angles,
+                                                  pitch_angles, output_width, output_height, fov_deg, lease=lease,
+                                                  devices=devices)
             except _engine.P2PError as e:
                 if e.code not in _ENCODER_FALLBACK_CODES:
                     raise
@@ -564,12 +498,9 @@ def process_single_image(input_image_path, output_dir, yaw_angles, pitch_angles,
         if jpeg:
             tasks = _save_files(files, base_name, output_dir, yaw_angles, pitch_angles, output_width, output_height,
                                 output_format, executor)
-        elif png:
-            tasks = _save_png(cv2, files, views, base_name, output_dir, yaw_angles, pitch_angles, output_width,
-                              output_height, output_format, executor)
         else:
             tasks = _save_views(cv2, views, base_name, output_dir, yaw_angles, pitch_angles, output_width,
-                                output_height, output_format, executor)
+                                output_height, output_format, executor, files)
         for future, yaw_angle in zip(tasks, yaw_angles):
             try:
                 future.result()
@@ -596,14 +527,17 @@ class _YawGroup:
 
 
 def _save_views(cv2, views, base_name, output_dir, yaw_angles, pitch_angles, output_width, output_height,
-                output_format, executor):
-    """Submit one encode task per view (reference file names, ref :275); returns one waitable per yaw."""
+                output_format, executor, files=None):
+    """Submit one task per view (reference file names, ref :275): ``files[k][i]`` when the device encoded it, else
+    ``cv2.imwrite`` of ``views[k, i]``; returns one waitable per yaw."""
 
     def save(k, i):
-        out_filename = (f"{base_name}_{output_width}x{output_height}_yaw_{yaw_angles[k]}"
-                        f"_pitch_{pitch_angles[i]}.{output_format}")
-        cv2.imwrite(str(output_dir / out_filename), views[k, i])
-        logging.debug(f"Saved {output_dir / out_filename}")
+        path = _out_path(output_dir, base_name, output_width, output_height, yaw_angles[k], pitch_angles[i], output_format)
+        if files is not None and files[k][i] is not None:
+            path.write_bytes(files[k][i])
+        else:
+            cv2.imwrite(str(path), views[k, i])
+        logging.debug(f"Saved {path}")
 
     return [_YawGroup([executor.submit(save, k, i) for i in range(len(pitch_angles))]) for k in range(len(yaw_angles))]
 
@@ -635,8 +569,8 @@ def process_image_batch(image_files, output_dir, yaw_angles, pitch_angles, outpu
         proj = get_projector(dev)
         # the host Huffman stage of a JPEG input runs on the worker thread: as many images in flight as there are workers
         n_in = max(1, min(int(inflight) if inflight else num_workers, proj.n_slots - 1))
-        jpeg_out = _is_jpeg(output_format)
-        if jpeg_out or str(output_format).lower() == "png":
+        jpeg_out, png_out = _is_jpeg(output_format), str(output_format).lower() == "png"
+        if jpeg_out or png_out:
             # every image in flight pins a file buffer of n_views x (W x H x 4 + 4096) bytes on its slot (plus the
             # encoders' device scratch): keep the total under a budget instead of running out of memory mid-folder
             per_slot = len(yaw_angles) * len(pitch_angles) * (W * H * 4 + 4096)
@@ -661,14 +595,15 @@ def process_image_batch(image_files, output_dir, yaw_angles, pitch_angles, outpu
             try:
                 futs = None
                 try:
-                    if jpeg_out:
-                        files_ = _project_jpeg(proj, src, yaw_angles, pitch_angles, W, H, fov_deg, lease=lease, devices=[])
-                        futs = _save_files(files_, f.stem, output_dir, yaw_angles, pitch_angles, W, H, output_format, writers)
-                    elif str(output_format).lower() == "png":
-                        files_, views = _project_png(proj, src, yaw_angles, pitch_angles, W, H, fov_deg, lease=lease,
-                                                     devices=[])
-                        futs = _save_png(cv2, files_, views, f.stem, output_dir, yaw_angles, pitch_angles, W, H,
-                                         output_format, writers)
+                    if jpeg_out or png_out:
+                        files_, views = _project_files("jpg" if jpeg_out else "png", proj, src, yaw_angles, pitch_angles,
+                                                       W, H, fov_deg, lease=lease, devices=[])
+                        if jpeg_out:
+                            futs = _save_files(files_, f.stem, output_dir, yaw_angles, pitch_angles, W, H, output_format,
+                                               writers)
+                        else:
+                            futs = _save_views(cv2, views, f.stem, output_dir, yaw_angles, pitch_angles, W, H, output_format,
+                                               writers, files_)
                 except _engine.P2PError as e:
                     if e.code not in _ENCODER_FALLBACK_CODES:
                         raise

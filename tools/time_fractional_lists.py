@@ -129,9 +129,7 @@ def main():
         return proj.encode_png(views.reshape(-1, H, W, 3)), views
 
     def new_files(fmt, src):
-        if fmt == "jpg":
-            return [f for per in front._project_jpeg(proj, src, YAWS, PITCHES, W, H, FOV, devices=[]) for f in per], None
-        files, views = front._project_png(proj, src, YAWS, PITCHES, W, H, FOV, devices=[])
+        files, views = front._project_files(fmt, proj, src, YAWS, PITCHES, W, H, FOV, devices=[])
         return [f for per in files for f in per], views
 
     src = front._open_image(src_file)
@@ -156,11 +154,11 @@ def main():
     for i in range(BATCH):
         (folder / f"p{i:02d}.jpg").write_bytes(data)
     files = sorted(folder.iterdir())
-    new_route = front._files_any_yaw
+    new_route = front._project_files
 
-    def old_route(proj_, fmt, src_, consts_, tables_, W_, H_, lease):
-        flat, views = old_files("png" if fmt == "png" else "jpg", src_)
-        return flat, views
+    def old_route(fmt, proj_, src_, yaws, pitches, W_, H_, fov, lease=None, devices=None):
+        flat, views = old_files(fmt, src_)
+        return [flat[k * n_p:(k + 1) * n_p] for k in range(len(yaws))], views
 
     for fmt in ("jpg", "png"):
         ts = {"old": [], "new": []}
@@ -171,13 +169,13 @@ def main():
                 if out.exists():
                     subprocess.run(["rm", "-rf", str(out)], check=True)
                 out.mkdir()
-                front._files_any_yaw = route
+                front._project_files = route
                 try:
                     t0 = time.perf_counter()
                     pkg.process_image_batch(files, out, YAWS, PITCHES, W, H, num_workers=8, output_format=fmt, fov_deg=FOV)
                     ts[name].append((time.perf_counter() - t0) * 1e3 / BATCH)
                 finally:
-                    front._files_any_yaw = new_route
+                    front._project_files = new_route
                 outs[name] = out
         same = all((outs["old"] / p.name).read_bytes() == p.read_bytes() for p in outs["new"].iterdir())
         same = same and len(list(outs["new"].iterdir())) == BATCH * len(YAWS) * n_p
