@@ -136,7 +136,6 @@ void p2p_destroy(p2p_ctx *ctx) {
     cudaFree(ctx->d_range);
     for (const p2p_ctx::JTab &t : ctx->jtabs) cudaFree(t.d);
     cudaFree(ctx->d_crc_table);
-    if (ctx->j_err_h) cudaFreeHost(ctx->j_err_h);
     cudaGetLastError();
     delete[] ctx->slots;
     delete ctx;

@@ -186,7 +186,6 @@ struct p2p_ctx {
     int jW = 0, jH = 0, jQ = 0;
     struct JTab { int W, H, Q; p2pjpeg::Tables *d; };
     std::vector<JTab> jtabs;            // one device copy per (size, quality) seen: a folder of mixed sizes never waits
-    int *j_err_h = nullptr, *j_err_d = nullptr;  // mapped: set by the encoder kernels when a file does not fit
     std::vector<RowRange> rows;   // memoised per geometry (the reference's pitch_mapping_cache key, ref :55-73)
     int *d_range = nullptr;
     long long launches = 0;

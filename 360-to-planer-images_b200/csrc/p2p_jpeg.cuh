@@ -445,8 +445,7 @@ struct BitSink {
 // thread per block: write the code bits at the block's bit offset
 __global__ void __launch_bounds__(256)
 jpeg_emit_kernel(const int16_t *__restrict__ coef, const uint32_t *__restrict__ offs, uint32_t *__restrict__ stream,
-                 const Tables *__restrict__ T, const Geometry G, const unsigned long long *__restrict__ total_bits,
-                 int *__restrict__ err) {
+                 const Tables *__restrict__ T, const Geometry G, const unsigned long long *__restrict__ total_bits) {
     __shared__ uint32_t s_ac[2][256];
     __shared__ uint32_t s_dc[2][16];
     for (int i = threadIdx.x; i < 512; i += blockDim.x) s_ac[i >> 8][i & 255] = T->ac[i >> 8][i & 255];
@@ -455,10 +454,7 @@ jpeg_emit_kernel(const int16_t *__restrict__ coef, const uint32_t *__restrict__ 
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     const int img = blockIdx.y;
     if (g >= G.n_blocks) return;
-    if (total_bits[img] > (unsigned long long)G.cap_bits_words * 32ull) {  // would not fit: report, write nothing
-        if (g == 0) atomicExch(err, 1);
-        return;
-    }
+    if (total_bits[img] > (unsigned long long)G.cap_bits_words * 32ull) return;  // would not fit: write nothing (size 0)
     const int mcu = g / 6, k = g - mcu * 6, t = (k < 4) ? 0 : 1;
     const int16_t *c = coef + ((size_t)img * G.n_blocks + g) * 64;
     const int p = pred_block(mcu, k);
@@ -541,7 +537,7 @@ jpeg_ffcount_kernel(const uint32_t *__restrict__ stream, uint32_t *__restrict__ 
 __global__ void __launch_bounds__(256)
 jpeg_stuff_kernel(const uint32_t *__restrict__ stream, const uint32_t *__restrict__ ffoff, uint8_t *__restrict__ out,
                   const Geometry G, const Tables *__restrict__ T, const unsigned long long *__restrict__ total_bits,
-                  const unsigned long long *__restrict__ total_ff, int *__restrict__ err) {
+                  const unsigned long long *__restrict__ total_ff) {
     const int img = blockIdx.y;
     const unsigned long long tb = total_bits[img];
     if (tb > (unsigned long long)G.cap_bits_words * 32ull) return;
@@ -549,10 +545,7 @@ jpeg_stuff_kernel(const uint32_t *__restrict__ stream, const uint32_t *__restric
     const unsigned long long chunks = (nbytes + 15) >> 4;
     const unsigned long long chunk = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (chunk >= chunks) return;
-    if ((unsigned long long)T->header_len + nbytes + total_ff[img] + 2ull > (unsigned long long)G.cap_out) {
-        if (chunk == 0) atomicExch(err, 1);
-        return;
-    }
+    if ((unsigned long long)T->header_len + nbytes + total_ff[img] + 2ull > (unsigned long long)G.cap_out) return;
     const uint8_t *s = reinterpret_cast<const uint8_t *>(stream + (size_t)img * G.cap_bits_words);
     const unsigned long long b0 = chunk << 4;
     uint8_t *dst = out + (size_t)img * G.cap_out + T->header_len + b0 + ffoff[(size_t)img * (G.cap_bits_words / 4) + chunk];
