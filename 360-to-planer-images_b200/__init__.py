@@ -13,6 +13,7 @@ from . import _lib
 
 _lib.load()  # fail loudly: no CPU fallback
 
+from . import folder_pool  # noqa: E402,F401
 from .engine import PinnedBuffer, Projector, host_assumptions, pitch_constants, warn_if_host_differs, yaw_table  # noqa: E402
 from .panorama_to_plane_pitch import (  # noqa: E402
     check_pitch,

@@ -22,7 +22,10 @@ class PitchConsts(C.Structure):
 class P2PError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__(f"p2p error {code}: {msg}")
-        self.code = code
+        self.code, self.msg = code, msg
+
+    def __reduce__(self):   # pickles with its code: a folder worker process's error is raised again in the caller
+        return type(self), (self.code, self.msg), self.__dict__
 
 
 # every symbol include/p2p.h declares: name -> (restype, argtypes)

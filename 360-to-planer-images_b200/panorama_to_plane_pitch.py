@@ -84,13 +84,18 @@ _png_formats = 0
 _host_checked = False
 
 
-def get_projector(device: int | None = None) -> _engine.Projector:
+def _check_host_once():
+    """Once per process: say so if this host does not meet the bit-exactness assumptions (no GPU involved)."""
     global _host_checked
+    if not _host_checked:
+        _host_checked = True
+        _engine.warn_if_host_differs(logging.getLogger())
+
+
+def get_projector(device: int | None = None) -> _engine.Projector:
     d = _default_device if device is None else int(device)
     with _projectors_lock:
-        if not _host_checked:   # once per process: say so if this host does not meet the bit-exactness assumptions
-            _host_checked = True
-            _engine.warn_if_host_differs(logging.getLogger())
+        _check_host_once()
         if d not in _projectors:
             _projectors[d] = _engine.Projector(d, n_slots=16)  # device buffers are allocated per slot on first use
             if _png_formats:
@@ -123,10 +128,11 @@ _DECLINED = (-6, -3, -5)
 class _JpegSource:
     """A JPEG or PNG panorama one of the device decoders handles, still as file bytes (the pixels will only exist on the GPU)."""
 
-    __slots__ = ("data", "Wp", "Hp", "path")
+    __slots__ = ("data", "Wp", "Hp", "path", "decoder")
 
     def __init__(self, data, dims, path):
         self.data, (self.Wp, self.Hp), self.path = data, dims, path
+        self.decoder = "device"   # "cv2.imread" once the device decoder has declined the file
 
 
 def _open_image(path):
@@ -165,6 +171,7 @@ def _decode_source(proj, src, slot=None, device_declined=False):
                 raise
     # the reference's own call: cv2.imread, not imdecode (for a truncated file libjpeg's file reader pads the scan and
     # returns an image where its memory reader gives up)
+    src.decoder = "cv2.imread"
     img = cv2.imread(str(src.path))
     if img is None:
         raise ValueError("Failed to decode image")
@@ -542,107 +549,163 @@ def _save_views(cv2, views, base_name, output_dir, yaw_angles, pitch_angles, out
     return [_YawGroup([executor.submit(save, k, i) for i in range(len(pitch_angles))]) for k in range(len(yaw_angles))]
 
 
+def run_device(dev, take, output_dir, yaw_angles, pitch_angles, W, H, num_workers, output_format, fov_deg, inflight=None,
+               host_wait=None, n_processes=1, confirm=None):
+    """The folder pipeline of one device (``process_image_batch``).  ``inflight`` host threads each take the next file
+    (``take()``; None when there is none left) and handle it start to finish on their own slot (stream): read (a JPEG or
+    PNG the device decoders handle stays file bytes, everything else goes to ``cv2.imread``), upload / decode, project,
+    read back or encode, hand the files to the pool of ``num_workers`` writer threads.  The library calls only hold the
+    context lock while they enqueue, so the threads overlap on the GPU and on the host.  ``confirm(file, decoder)`` is
+    called once a file's outputs are written: ``decoder`` is "device" when a device decoder read the panorama,
+    "cv2.imread" when cv2 did, None when the file could not be read.  ``n_processes``: processes running such a pipeline
+    on this host at once (for the sleeping-wait rule).  An exception a file raises outside the per-file error handling is
+    raised once every file has been taken."""
+    import cv2
+
+    output_dir = Path(output_dir)
+    num_workers = max(1, int(num_workers))
+    proj = get_projector(dev)
+    # the host Huffman stage of a JPEG input runs on the worker thread: as many images in flight as there are workers
+    n_in = max(1, min(int(inflight) if inflight else num_workers, proj.n_slots - 1))
+    jpeg_out, png_out = _is_jpeg(output_format), str(output_format).lower() == "png"
+    if jpeg_out or png_out:
+        # every image in flight pins a file buffer of n_views x (W x H x 4 + 4096) bytes on its slot (plus the
+        # encoders' device scratch): keep the total under a budget instead of running out of memory mid-folder
+        per_slot = len(yaw_angles) * len(pitch_angles) * (W * H * 4 + 4096)
+        budget = float(os.environ.get("P2P_PINNED_BUDGET_GB", "8")) * 2 ** 30
+        n_in = max(1, min(n_in, int(budget // max(1, per_slot))))
+    wait = host_wait if host_wait is not None else os.environ.get("P2P_HOST_WAIT")   # (the environment: for experiments)
+    if wait is None:
+        wait = 1 if (n_in + num_workers) * n_processes > (os.cpu_count() or 1) else 0
+    proj.set_option(_engine._lib.OPT_HOST_WAIT, int(bool(int(wait))))
+
+    def one(f, writers):
+        # the slot stays leased until this image's files are on disk (written straight from its page-locked buffer)
+        with contextlib.ExitStack() as lease:
+            return one_leased(f, writers, lease)
+
+    def one_leased(f, writers, lease):
+        logging.info(f"Loading image: {f}")
+        src = _open_image(f)
+        if src is None:
+            logging.error(f"Failed to read image: {f}")
+            return None
+        try:
+            futs = None
+            try:
+                if jpeg_out or png_out:
+                    files_, views = _project_files("jpg" if jpeg_out else "png", proj, src, yaw_angles, pitch_angles,
+                                                   W, H, fov_deg, lease=lease, devices=[])
+                    if jpeg_out:
+                        futs = _save_files(files_, f.stem, output_dir, yaw_angles, pitch_angles, W, H, output_format,
+                                           writers)
+                    else:
+                        futs = _save_views(cv2, views, f.stem, output_dir, yaw_angles, pitch_angles, W, H, output_format,
+                                           writers, files_)
+            except _engine.P2PError as e:
+                if e.code not in _ENCODER_FALLBACK_CODES:
+                    raise
+                logging.warning(f"Device encoder unavailable for {f} ({e}); writing with cv2.imwrite")
+            if futs is None:
+                views = _project(proj, src, yaw_angles, pitch_angles, W, H, fov_deg, devices=[])
+                futs = _save_views(cv2, views, f.stem, output_dir, yaw_angles, pitch_angles, W, H, output_format,
+                                   writers)
+        except Exception as e:
+            for yaw in yaw_angles:
+                logging.error(f"Error processing yaw_angle {yaw}: {e}")
+            return _read_by(src)
+        for fut, yaw in zip(futs, yaw_angles):
+            try:
+                fut.result()
+            except Exception as e:
+                logging.error(f"Error processing yaw_angle {yaw}: {e}")
+        return _read_by(src)
+
+    errors = []
+
+    def drain(writers):
+        while (f := take()) is not None:
+            try:
+                decoder = one(Path(f), writers)
+            except Exception as e:   # noqa: BLE001 - raised below, after the other files
+                errors.append(e)
+                continue
+            if confirm is not None:
+                confirm(f, decoder)
+
+    with ThreadPoolExecutor(max_workers=num_workers) as writers, ThreadPoolExecutor(max_workers=n_in) as workers:
+        for fut in [workers.submit(drain, writers) for _ in range(n_in)]:
+            fut.result()
+    if errors:
+        raise errors[0]
+
+
+def _read_by(src):
+    return src.decoder if isinstance(src, _JpegSource) else "cv2.imread"
+
+
+def _folder_worker_body(device, job, take, confirm):
+    """What a worker process of the folder pool (``folder_pool``) runs for one call: the caller's PNG decoder subset, then
+    the device pipeline over the files the caller hands out."""
+    global _host_checked
+    _host_checked = True    # the caller has checked this host (same interpreter and packages): warn once, not per worker
+    job = dict(job)
+    set_png_formats(job.pop("png_formats"))
+    run_device(device, take, confirm=confirm, **job)
+
+
 def process_image_batch(image_files, output_dir, yaw_angles, pitch_angles, output_width, output_height,
                         num_workers=4, output_format="png", fov_deg=90, devices=None, inflight=None, host_wait=None):
     """Directory front end (ref ``main`` :320-341 processes the files one after the other).
 
     Same files and names out as calling ``process_single_image`` per file, but ``inflight`` images (default: one per
-    worker, at most 15) are in flight at once, each on its own slot (stream) driven by its own host thread, while the writer pool saves earlier results.
-    ``devices`` shards the files round-robin over several GPUs (one pipeline per device, no data exchange).
+    worker, at most 15) are in flight at once, each on its own slot (stream) driven by its own host thread, while the
+    writer pool saves earlier results (``run_device``).
+    ``devices`` with two or more entries (an entry may repeat) and two or more files: one worker process per entry
+    (``folder_pool``, kept for later calls with the same list), each running this pipeline on its device with
+    ``num_workers // len(devices)`` writer threads; files go to whichever process asks first, so a mixed folder balances.
+    The workers start with ``spawn``: a script that makes such a call needs the ``if __name__ == "__main__":`` guard
+    (each worker imports the main script as ``__mp_main__``).  Such calls from several threads run one after the other.
     ``host_wait``: 1 = the in-flight threads sleep while they wait for the device, 0 = they spin (lowest latency, one busy
-    core each); default: sleep as soon as in-flight threads plus writers outnumber the host's cores.
+    core each); default: sleep as soon as in-flight threads plus writers of all processes outnumber the host's cores.
+    Returns {file: decoder} for every file handled: "device" when a device decoder read the panorama, "cv2.imread" when
+    cv2 did, None when it could not be read (logged).
     """
-    import cv2
-
     image_files = [Path(f) for f in image_files]
-    output_dir = Path(output_dir)
-    yaw_angles, pitch_angles = list(yaw_angles), list(pitch_angles)
     devices = [_default_device] if not devices else [int(d) for d in devices]
     num_workers = max(1, int(num_workers))
-    W, H = int(output_width), int(output_height)
-
-    def run_device(dev, files):
-        """Every image is handled start to finish by one of ``inflight`` host threads on its own slot (stream): read
-        (a JPEG the device decoder handles is Huffman-decoded on this thread, everything else by ``cv2.imread``),
-        upload / decode, project, read back or encode, hand the files to the writer pool.  The library calls only
-        hold the context lock while they enqueue, so the threads overlap on the GPU and on the host."""
-        proj = get_projector(dev)
-        # the host Huffman stage of a JPEG input runs on the worker thread: as many images in flight as there are workers
-        n_in = max(1, min(int(inflight) if inflight else num_workers, proj.n_slots - 1))
-        jpeg_out, png_out = _is_jpeg(output_format), str(output_format).lower() == "png"
-        if jpeg_out or png_out:
-            # every image in flight pins a file buffer of n_views x (W x H x 4 + 4096) bytes on its slot (plus the
-            # encoders' device scratch): keep the total under a budget instead of running out of memory mid-folder
-            per_slot = len(yaw_angles) * len(pitch_angles) * (W * H * 4 + 4096)
-            budget = float(os.environ.get("P2P_PINNED_BUDGET_GB", "8")) * 2 ** 30
-            n_in = max(1, min(n_in, int(budget // max(1, per_slot))))
-        wait = host_wait if host_wait is not None else os.environ.get("P2P_HOST_WAIT")   # (the environment: for experiments)
-        if wait is None:
-            wait = 1 if (n_in + num_workers) * len(devices) > (os.cpu_count() or 1) else 0
-        proj.set_option(_engine._lib.OPT_HOST_WAIT, int(bool(int(wait))))
-
-        def one(f, writers):
-            # the slot stays leased until this image's files are on disk (written straight from its page-locked buffer)
-            with contextlib.ExitStack() as lease:
-                one_leased(f, writers, lease)
-
-        def one_leased(f, writers, lease):
-            logging.info(f"Loading image: {f}")
-            src = _open_image(f)
-            if src is None:
-                logging.error(f"Failed to read image: {f}")
-                return
-            try:
-                futs = None
-                try:
-                    if jpeg_out or png_out:
-                        files_, views = _project_files("jpg" if jpeg_out else "png", proj, src, yaw_angles, pitch_angles,
-                                                       W, H, fov_deg, lease=lease, devices=[])
-                        if jpeg_out:
-                            futs = _save_files(files_, f.stem, output_dir, yaw_angles, pitch_angles, W, H, output_format,
-                                               writers)
-                        else:
-                            futs = _save_views(cv2, views, f.stem, output_dir, yaw_angles, pitch_angles, W, H, output_format,
-                                               writers, files_)
-                except _engine.P2PError as e:
-                    if e.code not in _ENCODER_FALLBACK_CODES:
-                        raise
-                    logging.warning(f"Device encoder unavailable for {f} ({e}); writing with cv2.imwrite")
-                if futs is None:
-                    views = _project(proj, src, yaw_angles, pitch_angles, W, H, fov_deg, devices=[])
-                    futs = _save_views(cv2, views, f.stem, output_dir, yaw_angles, pitch_angles, W, H, output_format,
-                                       writers)
-            except Exception as e:
-                for yaw in yaw_angles:
-                    logging.error(f"Error processing yaw_angle {yaw}: {e}")
-                return
-            for fut, yaw in zip(futs, yaw_angles):
-                try:
-                    fut.result()
-                except Exception as e:
-                    logging.error(f"Error processing yaw_angle {yaw}: {e}")
-
-        with ThreadPoolExecutor(max_workers=num_workers) as writers, ThreadPoolExecutor(max_workers=n_in) as workers:
-            for fut in [workers.submit(one, f, writers) for f in files]:
-                fut.result()
-
+    yaw_angles, pitch_angles = list(yaw_angles), list(pitch_angles)
     if not yaw_angles or not pitch_angles:
-        return
-    if len(devices) == 1:
-        run_device(devices[0], image_files)
-    else:
-        from . import shard
+        return {}
+    job = dict(output_dir=Path(output_dir), yaw_angles=yaw_angles, pitch_angles=pitch_angles, W=int(output_width),
+               H=int(output_height), output_format=output_format, fov_deg=fov_deg, inflight=inflight, host_wait=host_wait)
+    if len(devices) > 1 and len(image_files) > 1:
+        from . import folder_pool
 
-        with ThreadPoolExecutor(max_workers=len(devices)) as ex:
-            futs = [ex.submit(run_device, d, [image_files[i] for i in shard.shard_images(len(image_files), r, len(devices))])
-                    for r, d in enumerate(devices)]
-            for fu in futs:
-                fu.result()
+        n = len(devices)
+        job.update(num_workers=max(1, num_workers // n), n_processes=n, png_formats=_png_formats)
+        with _projectors_lock:
+            _check_host_once()
+        read = folder_pool.run_shared(devices, _folder_worker_body, job, image_files)
+    else:
+        read = {}
+        files, lock = iter(image_files), threading.Lock()
+
+        def take():
+            with lock:
+                return next(files, None)
+
+        run_device(devices[0], take, num_workers=num_workers, confirm=read.__setitem__, **job)
+    return {f: read[f] for f in image_files if f in read}
 
 
 def main(input_path, output_path, yaw_angles, pitch_angles, output_width, output_height,
          num_workers=None, output_format="png", fov_deg=90, enable_file_logging=False, devices=None):
-    """Process a single image or every image under a folder (ref :286-356)."""
+    """Process a single image or every image under a folder (ref :286-356).
+
+    ``devices`` (extra): several CUDA devices (a device may be listed twice).  A single image is split over them; a folder
+    runs one worker process per listed device (``process_image_batch``), started with ``spawn``, so a script that calls
+    ``main`` that way needs the ``if __name__ == "__main__":`` guard."""
     if num_workers is None:
         cpu_cores = os.cpu_count() or 1
         num_workers = max(1, int(cpu_cores * 0.9))
@@ -709,8 +772,9 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--enable_file_logging", action="store_true", help="Enable logging to a file.")
     p.add_argument("--device", type=int, default=0, help="CUDA device index (extra flag; default 0)")
     p.add_argument("--devices", type=int, nargs="+", default=None,
-                   help="several CUDA devices: the files of a folder are sharded round-robin, a single image is split "
-                        "by output row bands / views (extra flag)")
+                   help="several CUDA devices (a device may be listed twice): a folder runs one worker process per "
+                        "listed device, each taking the next file when it is free; a single image is split by output "
+                        "row bands / views (extra flag)")
     p.add_argument("--png_all_formats", action="store_true",
                    help="decode 16-bit, palette, 1/2/4-bit gray and interlaced PNG inputs on the GPU too (extra flag; same "
                         "pixels as cv2.imread)")
