@@ -94,6 +94,7 @@ SIGNATURES = {
     "p2p_coords": (_i, [_vp, _pcp, _i, _i, _i, _i, _f32p, _f32p]),
     "p2p_sample_with_maps": (_i, [_vp, _i, _i, _f32p, _f32p, _i, _i, _u8p]),
     "p2p_download_pano": (_i, [_vp, _i, _u8p, _sz]),
+    "p2p_debug_poison": (_i, [_vp, _i, _i]),
 }
 
 OPT_SAMPLER, OPT_WARP_W, OPT_YAWS_PER_THREAD, OPT_COUNT_LAUNCHES, OPT_IMAGES_PER_LAUNCH, OPT_MIRROR, OPT_INTERP, OPT_TRIG = 0, 1, 2, 3, 4, 5, 6, 7
@@ -104,6 +105,7 @@ OPT_SEAM_WRAP = 12
 OPT_HOST_WAIT = 13
 OPT_PNG_FORMATS = 14
 OPT_PNG_HOST_BLOCKS = 15
+OPT_POISON = 16
 
 _lib = None
 

@@ -202,6 +202,10 @@ int p2p_set_option(p2p_ctx *ctx, int key, int value) {
             if (value < 0 || value > 3) return fail(ctx, P2P_ERR_INVALID, "gpu_huffman must be 0 ... 3");
             ctx->opt_gpu_huffman = value;
             return P2P_OK;
+        case P2P_OPT_POISON:
+            if (value < -1 || value > 255) return fail(ctx, P2P_ERR_INVALID, "poison must be -1 (off) or a byte 0 ... 255");
+            ctx->opt_poison.store(value);
+            return P2P_OK;
 
         default:
             return fail(ctx, P2P_ERR_INVALID, "unknown option");
@@ -228,6 +232,7 @@ int p2p_get_option(p2p_ctx *ctx, int key, int *value) {
         case P2P_OPT_PNG_FORMATS: *value = ctx->opt_png_formats.load(); return P2P_OK;
         case P2P_OPT_GPU_HUFFMAN_COUNT: *value = (int)ctx->gpu_huffman_used; return P2P_OK;
         case P2P_OPT_PNG_HOST_BLOCKS: *value = (int)ctx->png_host_blocks.load(); return P2P_OK;
+        case P2P_OPT_POISON: *value = ctx->opt_poison.load(); return P2P_OK;
 
         default: return fail(ctx, P2P_ERR_INVALID, "unknown option");
     }
@@ -526,6 +531,64 @@ int p2p_download_pano(p2p_ctx *ctx, int slot, uint8_t *bgr_host, size_t row_stri
     if (e == cudaSuccess) e = wait_slot(ctx, s);
     cudaFree(d);
     if (e != cudaSuccess) return fail(ctx, P2P_ERR_CUDA, "p2p_download_pano", e);
+    return P2P_OK;
+}
+
+int p2p_debug_poison(p2p_ctx *ctx, int slot, int byte) {
+    if (!slot_ok(ctx, slot) || byte < 0 || byte > 255) return fail(ctx, P2P_ERR_INVALID, "bad slot or byte");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    Slot &s = ctx->slots[slot];
+    if (s.jd_run.pending) return fail(ctx, P2P_ERR_STATE, "a JPEG decode's Huffman verdict is still pending on the slot");
+    CK(cudaSetDevice(ctx->device));
+    CK(wait_slot(ctx, s));
+    const cudaStream_t st = s.stream;
+    const struct { void *p; size_t n; } scratch[] = {
+        {s.d_bgr, s.bgr_cap}, {s.d_out, s.out_cap}, {s.d_tab, s.tab_cap},
+        {s.j_coef, s.j_coef_cap}, {s.j_bits, s.j_bits_cap}, {s.j_stream, s.j_stream_cap}, {s.j_cnt, s.j_cnt_cap},
+        {s.j_out, s.j_out_cap}, {s.j_tot, s.j_tot_cap},
+        {s.pg_F, s.pg_F_cap}, {s.pg_tlen, s.pg_tlen_cap}, {s.pg_blk, s.pg_blk_cap}, {s.pg_info, s.pg_info_cap},
+        {s.pg_Z, s.pg_Z_cap}, {s.pg_sums, s.pg_sums_cap},
+        {s.jd_coef_d, s.jd_coef_d_cap}, {s.jd_planes, s.jd_planes_cap}, {s.jd_stream, s.jd_stream_cap},
+        {s.jd_states, s.jd_states_cap}, {s.jd_nblk, s.jd_nblk_cap}, {s.jd_tables, sizeof(p2pjdec::DevTables)},
+        {s.jd_dc, s.jd_dc_cap}, {s.jd_tiles, s.jd_tiles_cap}, {s.jd_tot_d, 4 * sizeof(unsigned long long)},
+        {s.jd_raw, s.jd_raw_cap}, {s.jd_dcnt, s.jd_dcnt_cap}, {s.jd_gate_d, 8 * sizeof(int)}, {s.jd_sub, s.jd_sub_cap},
+        {s.pd_zs, s.pd_zs_cap}, {s.pd_tab, s.pd_tab_cap}, {s.pd_raw, s.pd_raw_cap}, {s.pd_ref, s.pd_ref_cap},
+        {s.pd_match, s.pd_match_cap},
+    };
+    for (const auto &b : scratch)
+        if (b.p) CK(cudaMemsetAsync(b.p, byte, b.n, st));
+    // the panorama: packed rows row0 .. row1 hold it (columns 0 .. Wp: the wrap column included)
+    const bool held = s.valid && s.d_rgba;
+    if (s.d_rgba) {
+        uint8_t *base = reinterpret_cast<uint8_t *>(s.d_rgba);
+        const size_t row = (size_t)s.pitch_tex * 4;
+        const size_t a = held ? row * s.row0 : 0, b = held ? row * (s.row1 + 1) : 0;
+        if (a) CK(cudaMemsetAsync(base, byte, a, st));
+        if (s.rgba_cap > b) CK(cudaMemsetAsync(base + b, byte, s.rgba_cap - b, st));
+        if (held && s.pitch_tex > s.Wp + 1)
+            CK(cudaMemset2DAsync(base + a + (size_t)(s.Wp + 1) * 4, row, byte, (size_t)(s.pitch_tex - s.Wp - 1) * 4,
+                                 (size_t)(s.row1 - s.row0 + 1), st));
+    }
+    // the gather array and the folded planes hold rows row0 .. min(row1, Hp - 1) while they are current
+    const int k1 = (s.row1 < s.Hp - 1) ? s.row1 : s.Hp - 1;
+    if (s.arr) {
+        const bool keep = held && s.tex_current;
+        int rc = poison_array(ctx, s.surf, s.arrW, s.arrH, keep ? s.row0 : 1, keep ? k1 : 0, byte, st);
+        if (rc) return rc;
+    }
+    for (int c = 0; c < 3; ++c) {
+        if (!s.farr[c]) continue;
+        const bool keep = held && s.fold_current;
+        int rc = poison_array(ctx, s.fsurf[c], s.farrW, s.farrH, keep ? s.row0 : 1, keep ? k1 : 0, byte, st);
+        if (rc) return rc;
+    }
+    CK(wait_slot(ctx, s));
+    // pinned and mapped host buffers (no kernel of the slot runs any more)
+    if (s.jd_coef_h) memset(s.jd_coef_h, byte, s.jd_coef_h_cap);
+    if (s.pd_zs_h) memset(s.pd_zs_h, byte, s.pd_zs_h_cap);
+    if (s.pd_tab_h) memset(s.pd_tab_h, byte, s.pd_tab_h_cap);
+    if (s.j_sizes_h) memset(s.j_sizes_h, byte, (size_t)s.j_sizes_n * sizeof(unsigned long long));
+    if (s.jd_flags_h) memset(s.jd_flags_h, byte, sizeof(*s.jd_flags_h));
     return P2P_OK;
 }
 

@@ -179,6 +179,7 @@ struct p2p_ctx {
     int opt_gpu_huffman = 1;   // JPEG inputs without restart markers: Huffman decoding on the device
     std::atomic<int> opt_host_wait{0};   // 1: host threads sleep while they wait for a slot's stream (see wait_slot)
     std::atomic<int> opt_png_formats{0}; // PNG decoder subset (parse_png): 0 = 8-bit non-interlaced, 1 = every PNG format
+    std::atomic<int> opt_poison{-1};     // P2P_OPT_POISON: byte new buffers are filled with (-1: left as allocated)
     long long gpu_huffman_used = 0, gpu_huffman_fallback = 0;
     std::atomic<long long> png_host_blocks{0};   // dynamic PNG deflate blocks the chain walk measured because the search missed them
     uint32_t *d_crc_table = nullptr;    // CRC-32 table of the PNG encoder
@@ -222,6 +223,30 @@ int fail(p2p_ctx *ctx, int code, const char *what, cudaError_t e = cudaSuccess) 
         }                                                                 \
     } while (0)
 
+// P2P_OPT_POISON: fill a buffer the context has just allocated with the poison byte.  Device memory: on the legacy stream,
+// waited for (the slots' non-blocking streams do not wait for it); a debug facility, so the wait costs nothing that counts.
+int poison_new_device(p2p_ctx *ctx, void *p, size_t bytes) {
+    const int b = ctx->opt_poison.load(std::memory_order_relaxed);
+    if (b < 0) return P2P_OK;
+    CK(cudaMemset(p, b, bytes));
+    CK(cudaDeviceSynchronize());
+    return P2P_OK;
+}
+
+void poison_new_host(p2p_ctx *ctx, void *p, size_t bytes) {
+    const int b = ctx->opt_poison.load(std::memory_order_relaxed);
+    if (b >= 0) memset(p, b, bytes);
+}
+
+// every u32 texel of a Wa x Ha array outside rows keep0 .. keep1 := the poison byte (P2P_OPT_POISON, p2p_debug_poison);
+// not counted in P2P_OPT_COUNT_LAUNCHES, which must not depend on the poison
+int poison_array(p2p_ctx *ctx, cudaSurfaceObject_t surf, int Wa, int Ha, int keep0, int keep1, int byte, cudaStream_t st) {
+    if (byte < 0 || Wa <= 0 || Ha <= 0) return P2P_OK;
+    poison_surface_kernel<<<dim3((Wa + 255) / 256, Ha), 256, 0, st>>>(surf, Wa, keep0, keep1, 0x01010101u * (uint32_t)byte);
+    CK(cudaGetLastError());
+    return P2P_OK;
+}
+
 template <typename T>
 int ensure(p2p_ctx *ctx, T **ptr, size_t *cap, size_t bytes) {
     if (*cap >= bytes && *ptr) return P2P_OK;
@@ -237,7 +262,7 @@ int ensure(p2p_ctx *ctx, T **ptr, size_t *cap, size_t bytes) {
     CK(cudaMalloc(&p, bytes));
     *ptr = static_cast<T *>(p);
     *cap = bytes;
-    return P2P_OK;
+    return poison_new_device(ctx, p, bytes);
 }
 
 // for buffers whose size follows the CONTENT of a file (compressed scan length ...): grow with 50 % headroom, so that a
@@ -269,6 +294,7 @@ int ensure_file_sizes(p2p_ctx *ctx, Slot &s, int n) {
     s.j_sizes_h = nullptr;
     CK(cudaHostAlloc(reinterpret_cast<void **>(&s.j_sizes_h), (size_t)n * sizeof(unsigned long long),
                      cudaHostAllocMapped | cudaHostAllocPortable));
+    poison_new_host(ctx, s.j_sizes_h, (size_t)n * sizeof(unsigned long long));
     CK(cudaHostGetDevicePointer(reinterpret_cast<void **>(&s.j_sizes_d), s.j_sizes_h, 0));
     s.j_sizes_n = n;
     return P2P_OK;

@@ -239,6 +239,10 @@ class Projector:
     def sync(self, slot: int = -1):
         self._ck(self.lib.p2p_sync(self.ctx, slot))
 
+    def poison(self, slot: int, byte: int):
+        """Debug: fill everything ``slot`` does not hold with ``byte`` (``p2p_debug_poison``); waits for the slot."""
+        self._ck(self.lib.p2p_debug_poison(self.ctx, slot, int(byte)))
+
     # -- raw ABI calls ----------------------------------------------------------------------
     def upload(self, slot: int, pano: np.ndarray):
         pano = _as_u8_image(pano)

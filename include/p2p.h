@@ -103,6 +103,10 @@ typedef enum p2p_option {
     ,P2P_OPT_SEG_CHUNKS = 11       /* row-segment kernel: chunks of 32 pixel pairs per warp (default 4, 1..64) */
     ,P2P_OPT_PARTIAL_UPLOAD = 8    /* 1 (default): p2p_process_image copies only the panorama rows its views can
                                      touch (p2p_view_row_range) over PCIe; 0: always the whole panorama */
+    ,P2P_OPT_POISON = 16           /* debug: -1 (default) = off; 0..255: every buffer the context allocates from now on (device
+                                     scratch, panorama, gather arrays and folded planes, pinned and mapped host buffers) is
+                                     filled with this byte before its first use, so that a result which depends on memory no
+                                     call has written differs from the one of a run with another byte (see p2p_debug_poison) */
 
 } p2p_option;
 
@@ -380,6 +384,13 @@ int p2p_sample_with_maps(p2p_ctx *ctx, int slot, int yaw_shift, const float *U_h
                          const float *V_host, int W, int H, uint8_t *out_host);
 /* read back the packed panorama of a slot as BGR (checks upload / rotate) */
 int p2p_download_pano(p2p_ctx *ctx, int slot, uint8_t *bgr_host, size_t row_stride);
+/* fill everything the slot does not hold with `byte` (0..255), at full capacity: staging, output and table buffers, the
+ * scratch of every encoder and decoder (mapped flags and size arrays included), and the rows of the packed panorama, of
+ * its gather array and of its folded planes outside the rows the slot holds (plus the pitch padding of the held rows).
+ * What the slot holds and the context-wide caches are kept.  Waits for the slot's stream.  P2P_ERR_STATE while a JPEG
+ * decode's Huffman verdict is still pending on the slot.  Reuse of the slot then reads the byte wherever a call reads
+ * memory it has not written. */
+int p2p_debug_poison(p2p_ctx *ctx, int slot, int byte);
 
 #ifdef __cplusplus
 }
