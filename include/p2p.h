@@ -58,8 +58,10 @@ typedef enum p2p_option {
     P2P_OPT_YAWS_PER_THREAD = 2, /* 1..4 views sharing one coordinate evaluation (default 4) */
     P2P_OPT_COUNT_LAUNCHES = 3,  /* read-only via p2p_get_option: kernels launched so far (the fold of a panorama into
                                     its quarter-turn planes, like the refresh of its texture array, is not counted) */
-    P2P_OPT_IMAGES_PER_LAUNCH = 4, /* 1 (default), 2 or 4 resident panoramas share one launch (and one
-                                     coordinate evaluation) in p2p_project_batch */
+    P2P_OPT_IMAGES_PER_LAUNCH = 4, /* 2 or 4: consecutive resident panoramas of p2p_project_batch share one launch
+                                     (and one coordinate evaluation) of the generic kernel's multi-image variants.
+                                     1 (default): the row-segment kernel pairs same-stream resident panoramas of one
+                                     size by itself (their quarter-turn groups share launches) */
     P2P_OPT_MIRROR = 5            /* with the texture sampler and W % 8 == 0 the pixel pair (W/2 + t, W/2 - t) shares
                                      one coordinate evaluation.  2 (default): row-segment kernel - a warp walks a
                                      row segment, every output byte leaves in a packed 32-bit store, any flat view
